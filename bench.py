@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the placement hot path (BASELINE.json: "queries placed/s and k-mer lookups/s").
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--config 2|3|4|5] [--impl b200|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--config 2|3|4|5] [--impl b200|reference] [--dump-outputs DIR]
 
 A "step" is one pass of the hot path (extract + murmur3 + probe + count + descend) over one batch
 of synthetic reads of the named configuration (SURVEY.md section 8d; classeq2_b200/synth.py):
@@ -22,6 +22,13 @@ replicated and NO data-path collective (SURVEY.md 8e).
 `--impl reference` times the CPU restatement of the reference (oracle/classeq_oracle.cpp, all host
 cores) on a bounded sample of the same workload; the reference itself is Rust and cannot be built
 here (DESIGN.md).
+Every timed loop runs exactly K steps.
+
+`--dump-outputs DIR` writes, after the timed steps, the result arrays of the last kernel-resident step (the fields of
+`cls_result`, one element per read) as DIR/<field>.npy in float64, on a fixed, seeded sample of the reads whose indices
+are DIR/read_index.npy; the nested config-4 measurement adds DIR/config4_<field>.npy.  The workload is generated from
+fixed seeds, so two builds of the library run with the same arguments can be compared file by file.  Under torchrun
+rank 0 writes the results of its own reads.
 """
 from __future__ import annotations
 
@@ -47,6 +54,21 @@ NAMES = {2: "config2: synthetic 1,000-tip tree, 1 kb refs, 1M x 150 bp reads, in
 
 
 L2_NOTE = "256 MiB memset between steps of the GPU arm (outside the event pairs)"
+# --dump-outputs: reads kept of the main batch and of the nested config-4 batch; 9 float64 arrays each, 45 MiB in all
+DUMP_READS, DUMP_READS_CONFIG4, DUMP_SEED = 1 << 19, 1 << 17, 0
+
+
+def dump_outputs(directory: str, fields: dict, n_keep: int, prefix: str = "") -> None:
+    """Writes ``fields`` (equal-length per-read arrays) at a fixed, seeded sample of at most ``n_keep`` reads as
+    float64 .npy files, with the sampled read indices as ``<prefix>read_index.npy``."""
+    n = len(next(iter(fields.values())))
+    keep = np.arange(n) if n <= n_keep else np.sort(np.random.default_rng(DUMP_SEED).choice(n, n_keep, replace=False))
+    os.makedirs(directory, exist_ok=True)
+    for name, a in {"read_index": keep, **{k: v[keep] for k, v in fields.items()}}.items():
+        out = a.astype(np.float64)
+        if not np.array_equal(out.astype(a.dtype), a):       # node ids are uint64: exact only below 2^53
+            raise ValueError(f"--dump-outputs: {name} does not fit float64 exactly")
+        np.save(os.path.join(directory, f"{prefix}{name}.npy"), out)
 
 
 def common_config(config: int, n_total: int, world: int) -> dict:
@@ -346,6 +368,8 @@ def run_b200(args, rank, world, local_rank):
     # parity spot check of what was just timed (bit-exact against the CPU oracle on a sample)
     res = rb.fetch(stream.cuda_stream)
     status_hist = np.bincount(res.status, minlength=11).tolist()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {f: getattr(res, f) for f, _ in cq.engine.RESULT_DTYPES}, DUMP_READS)
 
     # ---- end to end through the C ABI with host buffers: `e2e` ----------------------------------------
     out = cq.BatchResult(n_local)
@@ -386,10 +410,9 @@ def run_b200(args, rank, world, local_rank):
             for _ in range(2):
                 mix.place_batch_into(bases, offsets, out2, params)
             t0 = time.perf_counter()
-            reps = max(1, args.steps // 2)
-            for _ in range(reps):
+            for _ in range(args.steps):
                 mix.place_batch_into(bases, offsets, out2, params)
-            dt = (time.perf_counter() - t0) / reps
+            dt = (time.perf_counter() - t0) / args.steps
             same2 = all((getattr(out2, f) == getattr(res, f)).all() for f, _ in cq.engine.RESULT_DTYPES)
             e2e_multi = {"value": n_local / dt, "unit": "reads/s", "n_devices": n_dev, "ms_per_step": dt * 1e3,
                          "equals_single_device": bool(same2),
@@ -498,7 +521,7 @@ def run_b200(args, rank, world, local_rank):
         dist.barrier()
         try:
             a5 = argparse.Namespace(**vars(args))
-            a5.config, a5.reads, a5.steps, a5.warmup, a5.device_build = 5, args.reads5 * world, max(2, min(args.steps, 3)), 2, True
+            a5.config, a5.reads, a5.warmup, a5.device_build, a5.dump_outputs = 5, args.reads5 * world, 2, True, None
             l5 = run_sharded(a5, rank, world, local_rank, embedded=True)
             if rank == 0 and l5:
                 c5 = {k: l5[k] for k in ("value", "unit", "ms_per_step", "steps", "warmup", "scaling", "lookups_per_s", "e2e", "config", "nvlink",
@@ -540,12 +563,11 @@ def run_config4_nested(args, local_rank):
     stream = torch.cuda.Stream(device=local_rank)
     flush = torch.empty(256 << 20, dtype=torch.uint8, device=f"cuda:{local_rank}")
     params = cq.PlaceParams()
-    steps = max(2, min(args.steps, 3))
     with torch.cuda.stream(stream):
         for _ in range(2):
             rb.place(params, stream.cuda_stream)
         ev = []
-        for i in range(steps):
+        for i in range(args.steps):
             flush.fill_(i)
             a, b = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
             a.record(stream)
@@ -556,6 +578,8 @@ def run_config4_nested(args, local_rank):
     ms = [a.elapsed_time(b) for a, b in ev]
     ms_per_step = float(np.mean(ms))
     res = rb.fetch(stream.cuda_stream)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {f: getattr(res, f) for f, _ in cq.engine.RESULT_DTYPES}, DUMP_READS_CONFIG4, "config4_")
     n_chk = min(len(lens), 2000)
     md = cpp_oracle.CppModel.from_flat(sm.flat)
     o = md.place_batch(bases[: int(offsets[n_chk])], offsets[: n_chk + 1], n_threads=os.cpu_count() or 1)
@@ -564,7 +588,7 @@ def run_config4_nested(args, local_rank):
     alg = algorithmic_bytes(lens)
     peak, _ = measured_peak()
     pc = probe_ceiling(int(info["table_bytes"]))
-    out = {"value": len(lens) / (ms_per_step / 1e3), "unit": "reads/s", "ms_per_step": ms_per_step, "steps": steps, "warmup": 2,
+    out = {"value": len(lens) / (ms_per_step / 1e3), "unit": "reads/s", "ms_per_step": ms_per_step, "steps": args.steps, "warmup": 2,
            "lookups_per_s": lookups / (ms_per_step / 1e3),
            "config": {"workload": NAMES[4], "reads": int(len(lens)), "mean_read_length": float(lens.mean()),
                       "index_entries": int(info["n_entries"]), "table_bytes": int(info["table_bytes"])},
@@ -662,16 +686,19 @@ def run_sharded(args, rank, world, local_rank, embedded=False):
     lookups_total = allred(float(lookups_local), dist.ReduceOp.SUM)
     value = reads_total / (ms_per_step / 1e3)
     res = [rb.fetch(st.cuda_stream) for rb in rbs]
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {f: np.concatenate([getattr(r, f) for r in res]) for f, _ in cq.engine.RESULT_DTYPES},
+                     DUMP_READS)
     line = None
 
     # end to end: host ASCII in, host arrays out, every sub-batch uploaded and fetched inside the timed region
     e2e_res = [sp.place(p, params) for p in parts]   # warm-up (first-use registration of the exchange buffers)
     barrier()
     t0 = time.perf_counter()
-    for _ in range(max(1, args.steps // 2)):
+    for _ in range(args.steps):
         e2e_res = [sp.place(p, params) for p in parts]
     torch.cuda.synchronize()
-    e2e_s = allred((time.perf_counter() - t0) / max(1, args.steps // 2), dist.ReduceOp.MAX)
+    e2e_s = allred((time.perf_counter() - t0) / args.steps, dist.ReduceOp.MAX)
 
     # parity: the replicated index on this GPU must give the very same arrays for EVERY read of EVERY sub-batch of this
     # rank (resident and end-to-end results alike); the counts are summed over the ranks
@@ -760,7 +787,13 @@ def main():
     ap.add_argument("--device-build", action="store_true",
                     help="set-up only: build the synthetic model's k-mer map on the GPU (cls_model_build_device) instead of the "
                          "host cores - the same arrays, outside every timed region")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the results of the last timed step (a fixed, seeded sample of the reads) as DIR/<field>.npy")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs: the reference arm places a timing-sized sample of the batch; dump the b200 arm")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))

@@ -86,7 +86,8 @@ def _fake_index_class(cq, cpp_oracle):
     return Index
 
 
-def test_default_flow_builds_the_whole_line_on_a_fake_device(monkeypatch, capsys):
+def _run_default_flow(monkeypatch, capsys, **overrides):
+    """`run_b200` on the fake device with shrunk models; returns the parsed line."""
     import torch
 
     import classeq2_b200 as cq
@@ -105,11 +106,18 @@ def test_default_flow_builds_the_whole_line_on_a_fake_device(monkeypatch, capsys
                         if device is not None else real_empty(*a, **k))
     monkeypatch.setattr(torch.Tensor, "pin_memory", lambda self: self)
     args = argparse.Namespace(gpus=1, steps=2, warmup=1, impl="b200", config=3, reads=3000, transport="p2p", cpu_seconds=0.3,
-                              no_config4=False, reads4=400, no_config5=False, reads5=1000, no_inprocess=False, device_build=False)
+                              no_config4=False, reads4=400, no_config5=False, reads5=1000, no_inprocess=False, device_build=False,
+                              dump_outputs=None)
+    for k, v in overrides.items():
+        setattr(args, k, v)
     bench.run_b200(args, 0, 1, 0)
     lines = [ln for ln in capsys.readouterr().out.splitlines() if ln.startswith("{")]
     assert len(lines) == 1
-    d = json.loads(lines[0])
+    return json.loads(lines[0])
+
+
+def test_default_flow_builds_the_whole_line_on_a_fake_device(monkeypatch, capsys):
+    d = _run_default_flow(monkeypatch, capsys)
     for key in ("metric", "value", "unit", "n_gpus", "steps", "warmup", "ms_per_step", "higher_is_better", "scaling", "vs_baseline", "dtype", "data",
                 "config", "e2e", "gpu_launches", "roofline", "cpu_baseline", "clocks", "parity", "config4"):
         assert key in d, key
@@ -130,7 +138,33 @@ def test_default_flow_builds_the_whole_line_on_a_fake_device(monkeypatch, capsys
     assert sum(d["status_histogram"]) == 3000 and np.isfinite(d["value"])
 
 
-def test_sharded_flow_builds_its_line_on_a_fake_device(monkeypatch, capsys):
+def test_default_flow_times_every_step_and_dumps_the_last_results(monkeypatch, capsys, tmp_path):
+    """--steps sets the timed steps of the nested config-4 measurement too; --dump-outputs writes the sampled results of
+    the last step, which equal the oracle's placements of the same seeded reads."""
+    from classeq2_b200 import engine
+    from oracle import cpp_oracle
+
+    assert 9 * 8 * (bench.DUMP_READS + bench.DUMP_READS_CONFIG4) <= 64 << 20
+    monkeypatch.setattr(bench, "DUMP_READS", 1000)
+    d = _run_default_flow(monkeypatch, capsys, steps=5, dump_outputs=str(tmp_path))
+    assert d["steps"] == 5 and len(d["step_ms"]) == 5 and d["gpu_launches"] == 15
+    assert d["config4"]["steps"] == 5 and len(d["config4"]["step_ms"]) == 5
+    fields = ["read_index"] + [f for f, _ in engine.RESULT_DTYPES]
+    assert sorted(p.name for p in tmp_path.iterdir()) == sorted(f"{p}{f}.npy" for p in ("", "config4_") for f in fields)
+    for prefix, config, n_reads, n_kept in (("", 3, 3000, 1000), ("config4_", 4, 400, 400)):
+        got = {f: np.load(tmp_path / f"{prefix}{f}.npy") for f in fields}
+        assert all(a.dtype == np.float64 and a.shape == (n_kept,) for a in got.values())
+        keep = got["read_index"].astype(np.int64)
+        assert (np.diff(keep) > 0).all() and keep[0] >= 0 and keep[-1] < n_reads
+        sm, bases, offsets, _, _ = bench.make_workload(config, 0, 1, n_reads)
+        md = cpp_oracle.CppModel.from_flat(sm.flat)
+        want = md.place_batch(bases, offsets, n_threads=4)
+        md.close()
+        for f, _ in engine.RESULT_DTYPES:
+            assert np.array_equal(got[f], want[f][keep].astype(np.float64)), (prefix, f)
+
+
+def test_sharded_flow_builds_its_line_on_a_fake_device(monkeypatch, capsys, tmp_path):
     """`run_sharded` (config 5; nested in every multi-GPU run of the default command) with world = 1: a stand-in for
     ``ShardedPlacer`` around the same oracle-backed index; the parity leg runs over every read of every sub-batch."""
     import torch
@@ -173,7 +207,8 @@ def test_sharded_flow_builds_its_line_on_a_fake_device(monkeypatch, capsys):
     real_empty = torch.empty
     monkeypatch.setattr(torch, "empty", lambda *a, device=None, **k: real_empty(*[min(x, 1 << 16) if isinstance(x, int) else x for x in a], **k))
     args = argparse.Namespace(gpus=1, steps=2, warmup=1, impl="b200", config=5, reads=2500, transport="p2p", cpu_seconds=0.3,
-                              no_config4=True, reads4=400, no_config5=True, reads5=1000, no_inprocess=True, device_build=False)
+                              no_config4=True, reads4=400, no_config5=True, reads5=1000, no_inprocess=True, device_build=False,
+                              dump_outputs=str(tmp_path))
     line = bench.run_sharded(args, 0, 1, 0)
     out = [ln for ln in capsys.readouterr().out.splitlines() if ln.startswith("{")]
     assert len(out) == 1 and json.loads(out[0])["value"] == line["value"]
@@ -181,5 +216,7 @@ def test_sharded_flow_builds_its_line_on_a_fake_device(monkeypatch, capsys):
     for key in ("metric", "value", "unit", "n_gpus", "ms_per_step", "scaling", "e2e", "gpu_launches", "roofline", "nvlink", "clocks", "config"):
         assert key in line, key
     assert sum(line["status_histogram"]) == 2500
+    assert np.array_equal(np.load(tmp_path / "read_index.npy"), np.arange(2500.0))        # every read: fewer than DUMP_READS
+    assert np.bincount(np.load(tmp_path / "status.npy").astype(np.int64), minlength=11).tolist() == line["status_histogram"]
     nested = bench.run_sharded(args, 0, 1, 0, embedded=True)        # the nested form: returned, not printed
     assert nested["parity"]["mismatching_fields"] == 0 and not [ln for ln in capsys.readouterr().out.splitlines() if ln.startswith("{")]

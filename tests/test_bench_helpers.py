@@ -43,3 +43,6 @@ def test_algorithmic_bytes_of_a_150_base_read():
 def test_help_and_argument_defaults():
     r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--help"], capture_output=True, text=True, timeout=120)
     assert r.returncode == 0 and "--gpus" in r.stdout and "--impl" in r.stdout and "--no-config4" in r.stdout
+    assert "--dump-outputs" in r.stdout
+    r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--steps", "0"], capture_output=True, text=True, timeout=120)
+    assert r.returncode == 2 and "--steps" in r.stderr
