@@ -126,6 +126,7 @@ PROTOTYPES = {
     "cls_index_create_shard": (C.c_int, [C.POINTER(ModelView), C.c_int, C.c_uint32, C.c_uint32, C.POINTER(C.c_void_p)]),
     "cls_index_create_multi": (C.c_int, [C.POINTER(ModelView), C.c_uint64, C.POINTER(C.c_void_p)]),
     "cls_index_create_devices": (C.c_int, [C.POINTER(ModelView), C.c_uint32, C.POINTER(C.c_int), C.POINTER(C.c_void_p)]),
+    "cls_index_create_sharded": (C.c_int, [C.POINTER(ModelView), C.c_uint32, C.POINTER(C.c_int), C.POINTER(C.c_void_p)]),
     "cls_routed_windows": (C.c_int, [C.c_void_p, C.c_void_p, u64p]),
     "cls_route_hashes": (C.c_int, [C.c_void_p, C.c_void_p, C.c_uint32, C.c_uint64, C.c_void_p, C.c_void_p, u64p, C.c_void_p]),
     "cls_shard_probe": (C.c_int, [C.c_void_p, C.c_void_p, C.c_uint64, C.c_void_p, C.c_void_p]),

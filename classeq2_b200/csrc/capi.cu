@@ -138,6 +138,37 @@ struct Workspace {
     bool in_use = false;
 };
 
+// One shard of a sharded handle (cls_index_create_sharded), in both of its roles in a sub-batch: HOME of a part of the
+// batch (its reads are packed, routed and placed on this shard's device) and OWNER of a slice of the table (it probes
+// the hashes every home sent it).  All buffers live on `device`, are allocated once and grow only when a larger
+// sub-batch needs them.
+struct ShardLane {
+    int device = 0;
+    cudaStream_t stream = nullptr;
+    cudaEvent_t route_ev = nullptr, probe_ev = nullptr;   // this home's hashes are in the owners' inboxes / this owner's replies are home
+    cudaEvent_t t_begin = nullptr, t_end = nullptr;       // device time of the sub-batch on this lane (cls_get_timing)
+    // owner side: n_shards segments of seg_cap hashes, segment h written by home h's route kernel (a peer store)
+    DevBuf inbox;
+    // home side: n_shards segments of seg_cap replies, segment o written by owner o's probe kernel; the window behind every
+    // slot; the run of every read in every owner's segment; the per-owner cursors (bytes 0..63) and the overflow flag (64)
+    DevBuf reply, slot_win, runs, state;
+    DevBuf d_words, d_descs, d_results, d_scratch, d_ascii, d_src, d_bad;
+    PinBuf h_words, h_descs, h_results, h_state, h_src, h_bad, h_ascii;
+    PackedLayout lay;
+    bool dev_pack = false;  // this home's reads of the current sub-batch were packed on the device
+    ShardLane() = default;
+    ShardLane(const ShardLane &) = delete;
+    ShardLane &operator=(const ShardLane &) = delete;
+    ~ShardLane() {
+        cudaSetDevice(device);
+        if (stream) { cudaStreamSynchronize(stream); cudaStreamDestroy(stream); }
+        for (cudaEvent_t e : {route_ev, probe_ev, t_begin, t_end}) if (e) cudaEventDestroy(e);
+        for (DevBuf *b : {&inbox, &reply, &slot_win, &runs, &state, &d_words, &d_descs, &d_results, &d_scratch, &d_ascii, &d_src, &d_bad})
+            b->release();
+        for (PinBuf *b : {&h_words, &h_descs, &h_results, &h_state, &h_src, &h_bad, &h_ascii}) b->release();
+    }
+};
+
 }  // namespace
 
 struct cls_index {
@@ -153,10 +184,21 @@ struct cls_index {
     // a multi-device handle (cls_index_create_devices): one full index per listed device; this front object
     // owns no device memory of its own, and every call that works on one device goes to replicas[0]
     std::vector<std::unique_ptr<cls_index>> replicas;
+    // a sharded handle (cls_index_create_sharded): shard s of the table on shards[s], its exchange state in lanes[s]; the
+    // calls on such a handle run one at a time (call_mu)
+    std::vector<std::unique_ptr<cls_index>> shards;
+    std::vector<std::unique_ptr<ShardLane>> lanes;
+    std::mutex call_mu;
+    struct ShardedCalls {   // the calls that take another path on such a handle (capi_sharded.cu)
+        int (*place_batch)(cls_index *, const cls_batch *, const cls_params *, cls_result *);
+        int (*place_resident)(cls_index *, cls_resident_batch *, const cls_params *, cudaStream_t);
+    };
+    const ShardedCalls *sharded = nullptr;
     cls_index() = default;
     cls_index(const cls_index &) = delete;
     cls_index &operator=(const cls_index &) = delete;
     ~cls_index() {   // also runs when cls_index_create fails half-way: nothing is leaked
+        lanes.clear();   // (before the shards: the lanes' streams may still run kernels that read the shards' tables)
         cudaSetDevice(device);
         for (auto &w : pool) {
             if (w->stream) { cudaStreamSynchronize(w->stream); cudaStreamDestroy(w->stream); }
@@ -977,14 +1019,9 @@ static int place_batch_one(cls_index *ix, const cls_batch *batch, const cls_para
     return place_batch_impl(ix, batch, params, result, n_devices_of_handle, false, &unused);
 }
 
-// Multi-device handle: the batch is cut into one contiguous part per replica (equal shares of the bases), every part
-// goes through the single-device pipeline on its own host thread (the packing loops of all parts share the one host
-// pool), and the result arrays are written in place - the reference's single process fanning out over its workers
-// (ports/cli/src/cmds/place_sequences.rs:125-156, place_sequences/mod.rs:123-126).
-static int place_batch_multi(cls_index *front, const cls_batch *batch, const cls_params *params, cls_result *result) {
-    const size_t nd = front->replicas.size();
+// Cut points of a batch into `nd` contiguous parts of equal shares of the bases (cut[0] = 0, cut[nd] = n).
+static std::vector<uint64_t> cut_by_bases(const cls_batch *batch, size_t nd) {
     const uint64_t n = batch->n_queries;
-    if (n && !batch->offsets) return fail(CLS_ERR_INVALID_ARGUMENT, "batch arrays are NULL");
     std::vector<uint64_t> cut(nd + 1, n);
     cut[0] = 0;
     if (n) {
@@ -996,21 +1033,39 @@ static int place_batch_multi(cls_index *front, const cls_batch *batch, const cls
             cut[d] = lo;
         }
     }
+    return cut;
+}
+
+// The caller's result arrays from query `a` on.
+static cls_result result_from(const cls_result *result, uint64_t a) {
+    cls_result r{};
+    r.status = result->status ? result->status + a : nullptr;
+    r.node_id = result->node_id ? result->node_id + a : nullptr;
+    r.one = result->one ? result->one + a : nullptr;
+    r.rest = result->rest ? result->rest + a : nullptr;
+    r.n_query_kmers = result->n_query_kmers ? result->n_query_kmers + a : nullptr;
+    r.n_matched = result->n_matched ? result->n_matched + a : nullptr;
+    r.n_root_matched = result->n_root_matched ? result->n_root_matched + a : nullptr;
+    r.iterations = result->iterations ? result->iterations + a : nullptr;
+    return r;
+}
+
+// Multi-device handle: the batch is cut into one contiguous part per replica (equal shares of the bases), every part
+// goes through the single-device pipeline on its own host thread (the packing loops of all parts share the one host
+// pool), and the result arrays are written in place - the reference's single process fanning out over its workers
+// (ports/cli/src/cmds/place_sequences.rs:125-156, place_sequences/mod.rs:123-126).
+static int place_batch_multi(cls_index *front, const cls_batch *batch, const cls_params *params, cls_result *result) {
+    const size_t nd = front->replicas.size();
+    const uint64_t n = batch->n_queries;
+    if (n && !batch->offsets) return fail(CLS_ERR_INVALID_ARGUMENT, "batch arrays are NULL");
+    const std::vector<uint64_t> cut = cut_by_bases(batch, nd);
     std::vector<int> rcs(nd, CLS_OK);
     std::vector<std::string> errs(nd);
     auto run = [&](size_t d) {
         const uint64_t a = cut[d], cnt = cut[d + 1] - a;
         if (cnt == 0) return;
         const cls_batch part{cnt, batch->bases, batch->offsets + a};   // offsets are absolute into `bases`
-        cls_result r{};
-        r.status = result->status ? result->status + a : nullptr;
-        r.node_id = result->node_id ? result->node_id + a : nullptr;
-        r.one = result->one ? result->one + a : nullptr;
-        r.rest = result->rest ? result->rest + a : nullptr;
-        r.n_query_kmers = result->n_query_kmers ? result->n_query_kmers + a : nullptr;
-        r.n_matched = result->n_matched ? result->n_matched + a : nullptr;
-        r.n_root_matched = result->n_root_matched ? result->n_root_matched + a : nullptr;
-        r.iterations = result->iterations ? result->iterations + a : nullptr;
+        cls_result r = result_from(result, a);
         try {
             rcs[d] = place_batch_one(front->replicas[d].get(), &part, params, &r, nd);
         } catch (const std::bad_alloc &) {
@@ -1047,12 +1102,14 @@ int cls_set_pack_mode(int mode) {
 
 int cls_place_batch(cls_index *ix, const cls_batch *batch, const cls_params *params, cls_result *result) try {
     if (!ix || !batch || !params || !result) return fail(CLS_ERR_INVALID_ARGUMENT, "NULL argument");
+    if (ix->sharded) return ix->sharded->place_batch(ix, batch, params, result);
     if (!ix->replicas.empty()) return place_batch_multi(ix, batch, params, result);
     return place_batch_one(ix, batch, params, result);
 } CLS_ABI_CATCH
 
 int cls_batch_upload(cls_index *ix, const cls_batch *batch, cls_resident_batch **out) try {
     if (!ix || !batch || !out) return fail(CLS_ERR_INVALID_ARGUMENT, "NULL argument");
+    if (!ix->shards.empty()) ix = ix->shards[0].get();       // a sharded handle: resident batches live on its first shard's device
     if (!ix->replicas.empty()) ix = ix->replicas[0].get();   // a multi-device handle: resident batches live on its first device
     *out = nullptr;
     CU_TRY(cudaSetDevice(ix->device));
@@ -1079,6 +1136,7 @@ int cls_batch_upload(cls_index *ix, const cls_batch *batch, cls_resident_batch *
 // ---- FASTA ingest on the device (SURVEY.md section 8f row 3; file_or_stdin.rs:76-116, sequence.rs:47-56) -----------
 int cls_fasta_upload(cls_index *ix, const uint8_t *text, uint64_t n_bytes, cls_resident_batch **out, cls_fasta_records *records) try {
     if (!ix || !out || !records || (n_bytes && !text)) return fail(CLS_ERR_INVALID_ARGUMENT, "NULL argument");
+    if (!ix->shards.empty()) ix = ix->shards[0].get();       // a sharded handle: resident batches live on its first shard's device
     if (!ix->replicas.empty()) ix = ix->replicas[0].get();   // a multi-device handle: resident batches live on its first device
     *out = nullptr;
     std::memset(records, 0, sizeof *records);
@@ -1208,6 +1266,7 @@ int cls_fasta_upload(cls_index *ix, const uint8_t *text, uint64_t n_bytes, cls_r
 
 int cls_place_resident(cls_index *ix, cls_resident_batch *rb, const cls_params *params, void *stream) try {
     if (!ix || !rb || !params) return fail(CLS_ERR_INVALID_ARGUMENT, "NULL argument");
+    if (ix->sharded) return ix->sharded->place_resident(ix, rb, params, (cudaStream_t)stream);
     if (!ix->replicas.empty()) ix = ix->replicas[0].get();   // a multi-device handle: resident batches live on its first device
     if (rb->device != ix->device) return fail(CLS_ERR_INVALID_ARGUMENT, "resident batch lives on another device");
     if (ix->n_shards > 1) return fail(CLS_ERR_INVALID_ARGUMENT, "this handle holds one shard of the index: use the routed calls");
@@ -1221,6 +1280,7 @@ int cls_place_resident(cls_index *ix, cls_resident_batch *rb, const cls_params *
 
 int cls_resident_fetch(cls_index *ix, cls_resident_batch *rb, void *stream, cls_result *result) try {
     if (!ix || !rb || !result) return fail(CLS_ERR_INVALID_ARGUMENT, "NULL argument");
+    if (!ix->shards.empty()) ix = ix->shards[0].get();       // a sharded handle: resident batches live on its first shard's device
     if (!ix->replicas.empty()) ix = ix->replicas[0].get();   // a multi-device handle: resident batches live on its first device
     CU_TRY(cudaSetDevice(ix->device));
     const size_t res_b = (size_t)rb->lay.n_device * sizeof(ResultRec);
@@ -1243,6 +1303,7 @@ uint64_t cls_resident_bytes(const cls_resident_batch *rb) {
 // ---- hash-sharded index: route -> (all-to-all) -> probe -> (all-to-all) -> place --------------------
 int cls_routed_windows(cls_index *ix, cls_resident_batch *rb, uint64_t *n_windows) try {
     if (!ix || !rb || !n_windows) return fail(CLS_ERR_INVALID_ARGUMENT, "NULL argument");
+    if (!ix->shards.empty()) return fail(CLS_ERR_INVALID_ARGUMENT, "a sharded handle routes internally: the routed calls take the handle of one shard");
     CU_TRY(cudaSetDevice(ix->device));
     if (!rb->d_runs.p) {
         const PackedLayout &lay = rb->lay;
@@ -1287,6 +1348,7 @@ static int route_hashes_impl(cls_index *ix, cls_resident_batch *rb, uint32_t n_s
 int cls_route_hashes(cls_index *ix, cls_resident_batch *rb, uint32_t n_shards, uint64_t seg_cap, void *d_send,
                      void *d_slot_win, uint64_t *counts_out, void *stream) try {
     if (!ix || !rb || !d_send || !d_slot_win || !counts_out) return fail(CLS_ERR_INVALID_ARGUMENT, "NULL argument");
+    if (!ix->shards.empty()) return fail(CLS_ERR_INVALID_ARGUMENT, "a sharded handle routes internally: the routed calls take the handle of one shard");
     if (n_shards == 0 || n_shards > kMaxShards) return fail(CLS_ERR_INVALID_ARGUMENT, "need 1 <= n_shards <= 8");
     uint64_t *seg[kMaxShards] = {nullptr};
     for (uint32_t o = 0; o < n_shards; ++o) seg[o] = (uint64_t *)d_send + (uint64_t)o * seg_cap;
@@ -1296,6 +1358,7 @@ int cls_route_hashes(cls_index *ix, cls_resident_batch *rb, uint32_t n_shards, u
 int cls_route_hashes_p2p(cls_index *ix, cls_resident_batch *rb, uint32_t n_shards, uint64_t seg_cap, void *const *d_segments,
                          void *d_slot_win, uint64_t *counts_out, void *stream) try {
     if (!ix || !rb || !d_segments || !d_slot_win || !counts_out) return fail(CLS_ERR_INVALID_ARGUMENT, "NULL argument");
+    if (!ix->shards.empty()) return fail(CLS_ERR_INVALID_ARGUMENT, "a sharded handle routes internally: the routed calls take the handle of one shard");
     if (n_shards == 0 || n_shards > kMaxShards) return fail(CLS_ERR_INVALID_ARGUMENT, "need 1 <= n_shards <= 8");
     uint64_t *seg[kMaxShards] = {nullptr};
     for (uint32_t o = 0; o < n_shards; ++o) {
@@ -1348,6 +1411,7 @@ int cls_peer_free(int device, void *d_ptr) try {
 
 int cls_shard_probe(cls_index *ix, const void *d_hashes, uint64_t n, void *d_replies, void *stream) try {
     if (!ix || (n && (!d_hashes || !d_replies))) return fail(CLS_ERR_INVALID_ARGUMENT, "NULL argument");
+    if (!ix->shards.empty()) return fail(CLS_ERR_INVALID_ARGUMENT, "a sharded handle routes internally: the routed calls take the handle of one shard");
     CU_TRY(cudaSetDevice(ix->device));
     cudaError_t e = launch_shard_probe(ix->dix, ix->shard, (const uint64_t *)d_hashes, n, d_replies, (cudaStream_t)stream);
     if (e != cudaSuccess) return fail(CLS_ERR_CUDA, std::string("probe kernel launch: ") + cudaGetErrorString(e));
@@ -1357,6 +1421,7 @@ int cls_shard_probe(cls_index *ix, const void *d_hashes, uint64_t n, void *d_rep
 int cls_place_routed(cls_index *ix, cls_resident_batch *rb, const void *d_replies, const void *d_slot_win,
                      uint32_t n_shards, uint64_t seg_cap, const cls_params *params, void *stream) try {
     if (!ix || !rb || !params || !d_replies || !d_slot_win) return fail(CLS_ERR_INVALID_ARGUMENT, "NULL argument");
+    if (!ix->shards.empty()) return fail(CLS_ERR_INVALID_ARGUMENT, "a sharded handle routes internally: the routed calls take the handle of one shard");
     if (n_shards == 0 || n_shards > kMaxShards) return fail(CLS_ERR_INVALID_ARGUMENT, "need 1 <= n_shards <= 8");
     if (!rb->d_runs.p) return fail(CLS_ERR_INVALID_ARGUMENT, "cls_route_hashes has not run on this batch");
     CU_TRY(cudaSetDevice(ix->device));
@@ -1414,6 +1479,7 @@ int cls_debug_kmer_hashes(int device, uint32_t k_size, const uint8_t *bases, uin
 int cls_debug_node_counts(cls_index *ix, const uint8_t *bases, uint64_t len, const cls_params *params, cls_level_count *rows,
                           uint64_t cap, uint64_t *n_rows, cls_result *result) try {
     if (!ix || !params || !n_rows || (len && !bases) || (cap && !rows)) return fail(CLS_ERR_INVALID_ARGUMENT, "NULL argument");
+    if (!ix->shards.empty()) return fail(CLS_ERR_INVALID_ARGUMENT, "this handle is sharded: no shard holds the whole table");
     if (!ix->replicas.empty()) ix = ix->replicas[0].get();   // a multi-device handle: resident batches live on its first device
     *n_rows = 0;
     if (ix->n_shards > 1) return fail(CLS_ERR_INVALID_ARGUMENT, "this handle holds one shard of the index");

@@ -70,6 +70,9 @@ cudaError_t launch_route(uint32_t k, const uint32_t *packed, const ReadDesc *rea
                          uint16_t *slot_win, uint2 *runs, unsigned long long *cursor, uint32_t *overflow, int sm_count, cudaStream_t stream);
 cudaError_t launch_shard_probe(const DeviceIndex &ix, uint32_t shard, const uint64_t *hashes, uint64_t n, void *replies,
                                cudaStream_t stream);
+// The same over a segment of `seg_cap` slots whose count is read on the device: min(*d_count, seg_cap) hashes.
+cudaError_t launch_shard_probe_counted(const DeviceIndex &ix, uint32_t shard, const uint64_t *hashes, uint64_t seg_cap,
+                                       const unsigned long long *d_count, void *replies, int sm_count, cudaStream_t stream);
 cudaError_t launch_place_routed(const DeviceIndex &ix, const PlaceParams &pp, const uint32_t *packed, const ReadDesc *reads,
                                 uint32_t first_read, uint32_t n_reads, ResultRec *results, const PlaceGeom &g,
                                 uint32_t n_shards, uint64_t seg_cap, const uint2 *runs, const uint16_t *slot_win, const void *replies,

@@ -154,10 +154,10 @@ __global__ void __launch_bounds__(256, 4) route_kernel(uint32_t k, const uint32_
 }
 
 // ---- stage 4: the owner answers ---------------------------------------------------------------
-__global__ void __launch_bounds__(256) shard_probe_kernel(DeviceIndex ix, uint32_t shard, const uint64_t *__restrict__ hashes,
-                                                          uint64_t n, ProbeReply *__restrict__ replies) {
-    __shared__ __align__(16) uint32_t stage[8][96];
-    const uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
+// Hashes [blk, blk + blockDim.x) of a segment of `n`: one thread per hash probes the local table shard.
+__device__ __forceinline__ void probe_block(const DeviceIndex &ix, uint32_t shard, const uint64_t *__restrict__ hashes, uint64_t n,
+                                            ProbeReply *__restrict__ replies, uint64_t blk, uint32_t (*stage)[96]) {
+    const uint64_t i = blk + threadIdx.x;
     const uint32_t lane = threadIdx.x & 31u, warp = threadIdx.x >> 5;
     ProbeReply rep{kEmpty, 0u, 0u};
     if (i < n) {
@@ -177,12 +177,35 @@ __global__ void __launch_bounds__(256) shard_probe_kernel(DeviceIndex ix, uint32
     // sectors - the destination may be a peer's memory across NVLink, where partial-sector stores cost a packet each)
     const uint64_t i0 = i - lane;
     const bool vector_ok = i0 + 32 <= n && ((reinterpret_cast<uintptr_t>(replies + i0) & 15u) == 0);
-    if (vector_ok) {
+    if (vector_ok) {   // (i0 is the same for the whole warp: a full warp of replies takes this path, or none of it)
         stage[warp][3 * lane] = rep.set_off; stage[warp][3 * lane + 1] = rep.slot; stage[warp][3 * lane + 2] = rep.code;
         __syncwarp();
         if (lane < 24) reinterpret_cast<uint4 *>(replies + i0)[lane] = reinterpret_cast<const uint4 *>(stage[warp])[lane];
+        __syncwarp();  // a later stride writes the stage again
     } else if (i < n) {
         replies[i] = rep;
+    }
+}
+
+// DEVICE_COUNT = false: `n` hashes, counted on the host; one thread per hash.  DEVICE_COUNT = true: the count is the sender's
+// cursor for this owner, read from device memory (a peer pointer into the sender's route state) and clamped to `n` =
+// seg_cap - a cursor that overflowed runs past the segment, and the clamp keeps the probe inside the inbox; the grid is
+// sized before the count is known and strides over the segment.
+template <bool DEVICE_COUNT>
+__global__ void __launch_bounds__(256) shard_probe_kernel(DeviceIndex ix, uint32_t shard, const uint64_t *__restrict__ hashes,
+                                                          uint64_t n, const unsigned long long *__restrict__ d_count,
+                                                          ProbeReply *__restrict__ replies) {
+    __shared__ __align__(16) uint32_t stage[8][96];
+    if constexpr (DEVICE_COUNT) {
+        __shared__ unsigned long long s_count;
+        if (threadIdx.x == 0) s_count = *d_count;   // one load per block (it may cross NVLink)
+        __syncthreads();
+        if (s_count < n) n = s_count;
+#pragma unroll 1
+        for (uint64_t blk = (uint64_t)blockIdx.x * blockDim.x; blk < n; blk += (uint64_t)gridDim.x * blockDim.x)
+            probe_block(ix, shard, hashes, n, replies, blk, stage);
+    } else {
+        probe_block(ix, shard, hashes, n, replies, (uint64_t)blockIdx.x * blockDim.x, stage);
     }
 }
 
@@ -306,7 +329,15 @@ cudaError_t launch_shard_probe(const DeviceIndex &ix, uint32_t shard, const uint
     if (n == 0) return cudaSuccess;
     const uint64_t blocks = (n + 255) / 256;
     if (blocks > 0x7FFFFFFFull) return cudaErrorInvalidConfiguration;
-    shard_probe_kernel<<<(uint32_t)blocks, 256, 0, stream>>>(ix, shard, hashes, n, reinterpret_cast<ProbeReply *>(replies));
+    shard_probe_kernel<false><<<(uint32_t)blocks, 256, 0, stream>>>(ix, shard, hashes, n, nullptr, reinterpret_cast<ProbeReply *>(replies));
+    return cudaGetLastError();
+}
+
+cudaError_t launch_shard_probe_counted(const DeviceIndex &ix, uint32_t shard, const uint64_t *hashes, uint64_t seg_cap,
+                                       const unsigned long long *d_count, void *replies, int sm_count, cudaStream_t stream) {
+    if (seg_cap == 0) return cudaSuccess;
+    const uint64_t blocks = std::min<uint64_t>((seg_cap + 255) / 256, (uint64_t)sm_count * 8);   // a full SM of 256-thread blocks, grid-stride
+    shard_probe_kernel<true><<<(uint32_t)blocks, 256, 0, stream>>>(ix, shard, hashes, seg_cap, d_count, reinterpret_cast<ProbeReply *>(replies));
     return cudaGetLastError();
 }
 

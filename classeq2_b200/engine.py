@@ -90,20 +90,29 @@ class Index:
     """A model serialised to one GPU (``cls_index_create``): upload once per model."""
 
     def __init__(self, model: Union[FlatModel, Tree, "_lib.ModelView"], device: int = 0, keepalive=None,
-                 shard: int = 0, n_shards: int = 1, devices=None, device_mask: Optional[int] = None):
+                 shard: int = 0, n_shards: int = 1, devices=None, device_mask: Optional[int] = None, sharded_devices=None):
         """``n_shards > 1``: this handle holds the k-mer table entries with ``(hash >> 61) % n_shards ==
         shard`` only (``cls_index_create_shard``); such a handle serves the routed calls of
         :mod:`classeq2_b200.parallel` and refuses ``place_batch``.
 
         ``devices`` (a list of CUDA devices, repeats allowed) or ``device_mask`` (bit d = device d, 0 = all visible):
         ONE handle over several GPUs (``cls_index_create_devices`` / ``cls_index_create_multi``): the index is
-        replicated, ``place_batch`` cuts every batch into one part per replica and runs them side by side."""
+        replicated, ``place_batch`` cuts every batch into one part per replica and runs them side by side.
+
+        ``sharded_devices`` (a list of 1 to 8 CUDA devices, repeats allowed): ONE handle over a HASH-SHARDED index
+        (``cls_index_create_sharded``): shard s of the k-mer table on ``sharded_devices[s]``, k-mers routed between the
+        devices inside the library.  ``place_batch``, ``upload``, ``upload_fasta`` and :func:`place_sequences` work on it,
+        for reads of up to 161 bases."""
         if isinstance(model, Tree):
             model = FlatModel.from_tree(model)
         view = model.view if hasattr(model, "view") else model
         self._keep = (model, keepalive)
         self._h = C.c_void_p()
-        if devices is not None:
+        if sharded_devices is not None:
+            devs = (C.c_int * len(sharded_devices))(*[int(d) for d in sharded_devices])
+            _lib.check(_lib.lib.cls_index_create_sharded(C.byref(view), len(sharded_devices), devs, C.byref(self._h)))
+            device = sharded_devices[0] if len(sharded_devices) else 0
+        elif devices is not None:
             devs = (C.c_int * len(devices))(*[int(d) for d in devices])
             _lib.check(_lib.lib.cls_index_create_devices(C.byref(view), len(devices), devs, C.byref(self._h)))
             device = devices[0] if len(devices) else 0

@@ -328,6 +328,30 @@ int cls_shard_probe(cls_index *index, const void *d_hashes, uint64_t n, void *d_
  *                          every reply straight into the memory of the GPU that asked;
  *   (barrier)  cls_place_routed on the local reply box.
  */
+/*
+ * The same hash-sharded index behind ONE handle of ONE process - the reference's CLI and watcher are single processes
+ * (ports/cli/src/cmds/place_sequences.rs:125-156): shard s (entries with (hash >> 61) % n_shards == s) on devices[s], the
+ * node-set records and the tree on every listed device.  1 <= n_shards <= 8; a device may be listed more than once
+ * (several shards on one GPU).  Peer access is enabled between every pair of distinct listed devices; a pair that
+ * cannot reach each other is CLS_ERR_UNSUPPORTED (there is no staged copy path).  On such a handle:
+ *   cls_place_batch      cuts the batch into one part per shard (equal shares of the bases; part s is placed at its
+ *                        HOME, devices[s]) and runs sub-batches of at most 2^19 reads per home, each as route -> probe ->
+ *                        place on one stream per shard, chained by events across devices: every home stores every hash
+ *                        straight into its owner's inbox (a peer store), every owner answers straight into the sender's
+ *                        reply box, every home places once every owner has answered.  The host waits once per
+ *                        sub-batch.  Exchange buffers are allocated once and grow with the sub-batch: at 2^19 reads of 150
+ *                        bases (k = 35) on eight shards, 3.1 GB per GPU.  A segment that overflows (a low-complexity read
+ *                        sends all its windows to one owner) runs that sub-batch again with an exact bound.
+ *                        cls_place_sequences goes through it.
+ *   cls_batch_upload, cls_fasta_upload, cls_resident_fetch   work on the first shard's device;
+ *   cls_place_resident   routes the resident batch from there to every owner, and WAITS for the placement;
+ *   cls_index_get_info   n_devices = n_shards, device = devices[0], n_entries / n_buckets / table_bytes summed;
+ *   cls_get_timing, cls_index_destroy as usual.
+ * Reads longer than 161 bases make the call CLS_ERR_UNSUPPORTED before anything runs.  The routed calls above and
+ * cls_debug_node_counts refuse the handle (CLS_ERR_INVALID_ARGUMENT).  Calls on one sharded handle from several host
+ * threads are correct and run one at a time.  Results are identical to those of a replicated index.
+ */
+int cls_index_create_sharded(const cls_model_view *model, uint32_t n_shards, const int *devices, cls_index **out);
 int cls_route_hashes_p2p(cls_index *index, cls_resident_batch *rb, uint32_t n_shards, uint64_t seg_cap,
                          void *const *d_segments, void *d_slot_win, uint64_t *counts_out, void *stream);
 int cls_peer_alloc(int device, uint64_t bytes, void **d_ptr, uint8_t ipc_handle[64]);
