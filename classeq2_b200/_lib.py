@@ -11,7 +11,7 @@ import ctypes as C
 import os
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
-# CLASSEQ_B200_LIB selects another build of the same library (kernel A/B experiments only)
+# CLASSEQ_B200_LIB selects another build of the same library (to compare two builds)
 LIB_PATH = os.environ.get("CLASSEQ_B200_LIB") or os.path.join(_HERE, "libclasseq_b200.so")
 
 CLS_OK = 0

@@ -124,12 +124,11 @@ struct PackedLayout {
 };
 
 struct Workspace {
-    cudaStream_t stream = nullptr, stream2 = nullptr, stream3 = nullptr;   // stream3: only the three-stream pipeline (CLS_PIPE=3)
-    cudaEvent_t ev[4] = {nullptr, nullptr, nullptr, nullptr};
+    cudaStream_t stream = nullptr, stream2 = nullptr, stream3 = nullptr;   // kernels; copies in; copies out
     std::vector<cudaEvent_t> chunk_ev;  // 4 per chunk: start, kernel start, kernel end, done
     PinBuf h_words, h_descs, h_results;
     DevBuf d_words, d_descs, d_results;
-    DevBuf d_scratch[2];                // scan -> descent hand-over of the chunk in flight on each stream
+    DevBuf d_scratch;                   // scan -> descent hand-over (every kernel runs on `stream`: stream order protects its reuse)
     // packing on the device (pack_kernels.cu): the batch's ASCII bases, where every read starts in them, invalid-base flags
     DevBuf d_ascii, d_src, d_bad;
     PinBuf h_src, h_bad, h_stage[2];    // h_stage: pinned staging ring for bases in pageable caller memory
@@ -201,14 +200,11 @@ struct cls_index {
         lanes.clear();   // (before the shards: the lanes' streams may still run kernels that read the shards' tables)
         cudaSetDevice(device);
         for (auto &w : pool) {
-            if (w->stream) { cudaStreamSynchronize(w->stream); cudaStreamDestroy(w->stream); }
-            if (w->stream2) { cudaStreamSynchronize(w->stream2); cudaStreamDestroy(w->stream2); }
-            if (w->stream3) { cudaStreamSynchronize(w->stream3); cudaStreamDestroy(w->stream3); }
+            for (cudaStream_t s : {w->stream, w->stream2, w->stream3}) { cudaStreamSynchronize(s); cudaStreamDestroy(s); }
             for (auto &e : w->chunk_ev) if (e) cudaEventDestroy(e);
-            for (auto &e : w->ev) if (e) cudaEventDestroy(e);
             w->h_words.release(); w->h_descs.release(); w->h_results.release();
             w->d_words.release(); w->d_descs.release(); w->d_results.release();
-            w->d_scratch[0].release(); w->d_scratch[1].release();
+            w->d_scratch.release();
             for (auto &e : w->stage_ev) if (e) cudaEventDestroy(e);
             w->d_ascii.release(); w->d_src.release(); w->d_bad.release();
             w->h_src.release(); w->h_bad.release(); w->h_stage[0].release(); w->h_stage[1].release();
@@ -445,14 +441,11 @@ Workspace *acquire_ws(cls_index *ix) {
     for (auto &w : ix->pool)
         if (!w->in_use) { w->in_use = true; return w.get(); }
     auto w = std::make_unique<Workspace>();
-    bool ok = cudaStreamCreateWithFlags(&w->stream, cudaStreamNonBlocking) == cudaSuccess &&
-              cudaStreamCreateWithFlags(&w->stream2, cudaStreamNonBlocking) == cudaSuccess;
-    for (auto &e : w->ev)
-        if (ok) ok = cudaEventCreate(&e) == cudaSuccess;
+    bool ok = true;
+    for (cudaStream_t *s : {&w->stream, &w->stream2, &w->stream3})
+        if (ok) ok = cudaStreamCreateWithFlags(s, cudaStreamNonBlocking) == cudaSuccess;
     if (!ok) {   // nothing half-made is left behind
-        if (w->stream) cudaStreamDestroy(w->stream);
-        if (w->stream2) cudaStreamDestroy(w->stream2);
-        for (auto &e : w->ev) if (e) cudaEventDestroy(e);
+        for (cudaStream_t s : {w->stream, w->stream2, w->stream3}) if (s) cudaStreamDestroy(s);
         return nullptr;
     }
     w->in_use = true;
@@ -475,11 +468,8 @@ struct WsGuard {
     bool clean = false;
     ~WsGuard() {
         if (!w) return;
-        if (!clean) {
-            if (w->stream) cudaStreamSynchronize(w->stream);
-            if (w->stream2) cudaStreamSynchronize(w->stream2);
-            if (w->stream3) cudaStreamSynchronize(w->stream3);
-        }
+        if (!clean)
+            for (cudaStream_t s : {w->stream, w->stream2, w->stream3}) cudaStreamSynchronize(s);
         release_ws(ix, w);
     }
 };
@@ -516,13 +506,6 @@ static int upload_index(const HostIndex &h, int device, uint32_t shard, uint32_t
     cudaDeviceProp prop;
     CU_TRY(cudaGetDeviceProperties(&prop, device));
     if (prop.major < 10) return fail(CLS_ERR_CUDA, "this library only carries sm_100a code; device is sm_" + std::to_string(prop.major) + std::to_string(prop.minor));
-
-    // EXPERIMENT (CLS_L2_FETCH=32|64|128): the probes are random 32-byte sectors; a larger L2 fetch granularity
-    // reads neighbours that nobody asks for (a hint the platform may ignore)
-    if (const char *gr = getenv("CLS_L2_FETCH")) {
-        const size_t want = (size_t)atoi(gr);
-        if (want) (void)cudaDeviceSetLimit(cudaLimitMaxL2FetchGranularity, want);
-    }
     auto ix = std::make_unique<cls_index>();
     ix->device = device;
     ix->sm_count = prop.multiProcessorCount;
@@ -786,8 +769,8 @@ static int place_batch_impl(cls_index *ix, const cls_batch *batch, const cls_par
                 }
         }
     }
-    // Chunks of every length class go through pack (host threads) -> H2D -> kernel -> D2H on two
-    // alternating streams: chunk c+1 is packed and copied while chunk c is on the SMs, and the
+    // Chunks of every length class go through pack (host threads) -> H2D -> kernel -> D2H on three
+    // streams: chunk c+1 is packed and copied while chunk c is on the SMs, and the
     // results of finished chunks are scattered to the caller's arrays while later chunks run.
     struct Chunk { uint32_t first, count, max_len; };
     std::vector<Chunk> chunks;
@@ -796,24 +779,23 @@ static int place_batch_impl(cls_index *ix, const cls_batch *batch, const cls_par
     static const uint64_t kChunkEnv = [] { const char *e = getenv("CLS_CHUNK_MBASES"); return (uint64_t)(e ? atoi(e) : 0) << 20; }();
     const uint64_t total_bases = batch->n_queries ? batch->offsets[batch->n_queries] - batch->offsets[0] : 0;
     const uint64_t kChunkBases = kChunkEnv ? kChunkEnv : std::max<uint64_t>((uint64_t)24 << 20, total_bases / 12);
+    // the very first chunk holds a quarter of `per` reads so that the GPU starts early; later ones grow up to twice `per`
+    // (fewer launch tails).  (x 1.5 per chunk: the host packs chunk c + 1 while the GPU places chunk c, at about half the
+    // GPU's time per read - doubling the chunks left the GPU waiting at every step of the ramp: 54.8 against 52.2 ms per
+    // 10 M reads, profiles/r2b)
+    constexpr uint64_t kFirstChunkDiv = 4, kChunkGrowthPct = 150, kChunkRampMax = 2;
     for (const LengthClass &c : lay.classes) {
         const uint64_t per = std::max<uint64_t>(4096, kChunkBases / std::max<uint32_t>(c.max_len, 1));
-        // the very first chunks are small so that the GPU starts early; later ones grow (fewer launch tails)
-        static const int ramp = [] { const char *e = getenv("CLS_CHUNK_RAMP"); return e ? atoi(e) : 2; }();
-        // (x 1.5 per chunk: the host packs chunk c + 1 while the GPU places chunk c, at about half the GPU's time per read -
-        // doubling the chunks left the GPU waiting at every step of the ramp: 54.8 against 52.2 ms per 10 M reads, profiles/r2b)
-        static const int growth = [] { const char *e = getenv("CLS_CHUNK_GROWTH"); return e && atoi(e) > 100 ? atoi(e) : 150; }();
-        static const int first_div = [] { const char *e = getenv("CLS_CHUNK_FIRST"); return e && atoi(e) > 0 ? atoi(e) : 4; }();
-        uint64_t a = 0, step = (ramp && chunks.empty()) ? std::max<uint64_t>(4096, per / first_div) : per;
+        uint64_t a = 0, step = chunks.empty() ? std::max<uint64_t>(4096, per / kFirstChunkDiv) : per;
         while (a < c.count) {
             const uint64_t n = std::min<uint64_t>(step, c.count - a);
             chunks.push_back(Chunk{(uint32_t)(c.first + a), (uint32_t)n, c.max_len});
             a += n;
-            if (ramp) step = std::min<uint64_t>(step * growth / 100, per * (uint64_t)ramp);
+            step = std::min<uint64_t>(step * kChunkGrowthPct / 100, per * kChunkRampMax);
         }
         // ... and the very last ones shrink again: what follows the last kernel (its results' way back, their scatter) is
         // exposed, and is as long as the last chunk
-        if (ramp && &c == &lay.classes.back())
+        if (&c == &lay.classes.back())
             for (int r = 0; r < 3 && chunks.back().count > std::max<uint64_t>(8192, per / 4); ++r) {
                 Chunk last = chunks.back();
                 const uint32_t half = last.count / 2;
@@ -842,10 +824,17 @@ static int place_batch_impl(cls_index *ix, const cls_batch *batch, const cls_par
         }
         return CLS_OK;
     };
+    // Copies in, kernels and copies out run on THREE streams chained by events, so that the kernels of consecutive
+    // chunks never share the SMs (with everything of a chunk on one of two alternating streams the scan kernel of chunk
+    // c + 1 starts while the descent kernel of chunk c still holds warp slots: 8.13 against 7.70 ms per 1 M reads end to
+    // end, profiles/r2a).
+    // With device packing the bases go up in pieces that do not end where the chunks end: a piece copied for chunk c holds
+    // the first bases of chunk c + 1, so all copies in have to share ONE stream for a chunk's pack kernel to wait for them.
+    cudaStream_t st_in = w->stream2, st_k = w->stream, st_out = w->stream3;
     // device packing: the caller's bases go up in input order, piece by piece, on the copy stream; a chunk's pack kernel
     // runs once everything up to the last base of its reads is there (one length class: chunk c needs just its own range)
     uint64_t uploaded = 0, piece_no = 0;
-    auto upload_to = [&](uint64_t end, cudaStream_t st_in) -> int {
+    auto upload_to = [&](uint64_t end) -> int {
         while (uploaded < end) {
             const uint64_t n = std::min(kPiece, end - uploaded);
             const uint8_t *src = batch->bases + base0 + uploaded;
@@ -865,17 +854,6 @@ static int place_batch_impl(cls_index *ix, const cls_batch *batch, const cls_par
         }
         return CLS_OK;
     };
-    // Copies in, kernels and copies out run on THREE streams chained by events, so that the kernels of consecutive
-    // chunks never share the SMs (with everything of a chunk on one of two alternating streams the scan kernel of chunk
-    // c + 1 starts while the descent kernel of chunk c still holds warp slots: 8.13 against 7.70 ms per 1 M reads end to
-    // end, profiles/r2a).  CLS_PIPE=2 selects the two-stream pipeline (A/B).
-    // With device packing the bases go up in pieces that do not end where the chunks end: a piece copied for chunk c holds
-    // the first bases of chunk c + 1, so all copies in have to share ONE stream for a chunk's pack kernel to wait for them
-    // (the two-stream pipeline let it read bases another stream was still copying: found by ThreadSanitizer on the fake
-    // runtime with asynchronous streams, tests/test_capi_fake.py) - device packing always takes the three-stream pipeline.
-    static const bool pipe3_env = [] { const char *e = getenv("CLS_PIPE"); return !(e && atoi(e) == 2); }();
-    const bool pipe3 = pipe3_env || dev_pack;
-    if (pipe3 && !w->stream3) CU_TRY(cudaStreamCreateWithFlags(&w->stream3, cudaStreamNonBlocking));
     for (size_t ci = 0; ci < chunks.size(); ++ci) {
         if (fast) {   // the layout of this chunk's reads, just in time
             const double tq = now_ms();
@@ -892,8 +870,6 @@ static int place_batch_impl(cls_index *ix, const cls_batch *batch, const cls_par
             tm.pack_ms += now_ms() - tq;
         }
         const Chunk &c = chunks[ci];
-        cudaStream_t st = (ci & 1) ? w->stream2 : w->stream;                 // default: everything of a chunk on one of two streams
-        cudaStream_t st_in = pipe3 ? w->stream2 : st, st_k = pipe3 ? w->stream : st, st_out = pipe3 ? w->stream3 : st;
         cudaEvent_t *ev = &w->chunk_ev[4 * ci];
         const double tp = now_ms();
         const size_t w0 = word_off[c.first], w1 = word_off[c.first + c.count];
@@ -923,7 +899,7 @@ static int place_batch_impl(cls_index *ix, const cls_batch *batch, const cls_par
             // (just-in-time plan: the device order is the input order, a chunk's bases are one range - the ranges of
             // host-packed chunks are never sent)
             if (fast && uploaded < h_src[c.first]) uploaded = h_src[c.first];
-            rc = upload_to(need.load(), st_in);
+            rc = upload_to(need.load());
             if (rc != CLS_OK) return rc;
             tm.pack_ms += now_ms() - tp;
             CU_TRY(cudaMemcpyAsync(d_src + c.first, h_src + c.first, (size_t)c.count * 8, cudaMemcpyHostToDevice, st_in));
@@ -938,30 +914,30 @@ static int place_batch_impl(cls_index *ix, const cls_batch *batch, const cls_par
         CU_TRY(cudaMemcpyAsync(d_descs + c.first, h_descs + c.first, (size_t)c.count * sizeof(ReadDesc), cudaMemcpyHostToDevice, st_in));
         tm.h2d_bytes += (uint64_t)c.count * sizeof(ReadDesc);
         CU_TRY(cudaEventRecord(ev[1], st_in));
-        if (pipe3) CU_TRY(cudaStreamWaitEvent(st_k, ev[1], 0));
+        CU_TRY(cudaStreamWaitEvent(st_k, ev[1], 0));
         if (dev_c) {
             cudaError_t pe = launch_ascii_pack(d_ascii, d_src, d_descs, c.first, c.count, c.max_len, d_words, d_bad, st_k);
             if (pe != cudaSuccess) return fail(CLS_ERR_CUDA, std::string("pack kernel launch: ") + cudaGetErrorString(pe));
             tm.kernel_launches += 1;
         }
         PlaceGeom g = make_place_geom(c.max_len, ix->dix.k_size, ix->dix.max_fanout);
-        DevBuf &scratch = w->d_scratch[ci & 1];  // stream order protects its reuse by the chunk after next
-        if (pipe3 && place_scratch_bytes(c.count, c.max_len, ix->dix.k_size, ix->dix.max_fanout) > scratch.cap && scratch.p)
-            CU_TRY(cudaStreamSynchronize(st_k));   // growing a scratch buffer frees it: nothing on the kernel stream may still use it
-        CU_TRY(scratch.reserve(place_scratch_bytes(c.count, c.max_len, ix->dix.k_size, ix->dix.max_fanout)));
+        DevBuf &scratch = w->d_scratch;
+        const size_t scratch_b = place_scratch_bytes(c.count, c.max_len, ix->dix.k_size, ix->dix.max_fanout);
+        if (scratch_b > scratch.cap && scratch.p)
+            CU_TRY(cudaStreamSynchronize(st_k));   // growing the scratch buffer frees it: nothing on the kernel stream may still use it
+        CU_TRY(scratch.reserve(scratch_b));
         uint32_t nl = 0;
         cudaError_t e = launch_place(ix->dix, pp, d_words, d_descs, c.first, c.count, d_res, g, ix->sm_count, st_k,
                                      scratch.p, scratch.cap, &nl);
         if (e != cudaSuccess) {
-            cudaStreamSynchronize(w->stream); cudaStreamSynchronize(w->stream2);
-            if (w->stream3) cudaStreamSynchronize(w->stream3);
+            for (cudaStream_t s : {st_in, st_k, st_out}) cudaStreamSynchronize(s);
             if (e == cudaErrorInvalidConfiguration)
                 return fail(CLS_ERR_UNSUPPORTED, "query too long (or tree fan-out too large) for the per-read shared-memory tables");
             return fail(CLS_ERR_CUDA, std::string("place kernel launch: ") + cudaGetErrorString(e));
         }
         tm.kernel_launches += nl;
         CU_TRY(cudaEventRecord(ev[2], st_k));
-        if (pipe3) CU_TRY(cudaStreamWaitEvent(st_out, ev[2], 0));
+        CU_TRY(cudaStreamWaitEvent(st_out, ev[2], 0));
         CU_TRY(cudaMemcpyAsync(h_res + c.first, d_res + c.first, (size_t)c.count * sizeof(ResultRec), cudaMemcpyDeviceToHost, st_out));
         tm.d2h_bytes += (uint64_t)c.count * sizeof(ResultRec);
         if (dev_c) {
@@ -1003,9 +979,8 @@ static int place_batch_one(cls_index *ix, const cls_batch *batch, const cls_para
                            size_t n_devices_of_handle = 1) {
     if (ix->n_shards > 1) return fail(CLS_ERR_INVALID_ARGUMENT, "this handle holds one shard of the index: use the routed calls");
     // batches that look like short reads (k = 35, mean length within the one-warp geometry) try the just-in-time plan
-    static const bool no_fast = getenv("CLS_NO_FASTPLAN") != nullptr;
     const uint64_t n = batch->n_queries;
-    bool fast = !no_fast && ix->dix.k_size == 35 && n >= 1 && n < 0xFFFFFFFFull && batch->offsets && batch->bases;
+    bool fast = ix->dix.k_size == 35 && n >= 1 && n < 0xFFFFFFFFull && batch->offsets && batch->bases;
     if (fast) {
         const uint64_t o0 = batch->offsets[0], o1 = batch->offsets[n];
         fast = o1 >= o0 && (o1 - o0) >= n * 35 && (o1 - o0) <= n * (uint64_t)kFastMaxLen;

@@ -1340,9 +1340,6 @@ namespace {
 // The descent kernel of the short-read path (at most kPairCap pairs per read).  A warp takes 16 consecutive reads from the
 // global counter, sorts them into size classes by their number of pairs and runs four reads of at most 8 pairs, or two
 // of at most 16, side by side (finish_group); the others - and whatever finish_group hands back - go one read per warp.
-#ifndef CLS_DESCEND_GROUPS
-#define CLS_DESCEND_GROUPS 1
-#endif
 template <int G>
 __device__ __forceinline__ uint32_t run_groups(const DeviceIndex &ix, const PlaceParams &pp, const ScanOut &so, uint32_t first_read,
                                                ResultRec *__restrict__ results, uint32_t mask, uint32_t my_r, uint2 my_me) {
@@ -1447,11 +1444,6 @@ PlaceGeom make_place_geom(uint32_t max_len, uint32_t k, uint32_t max_fanout) {
     return g;
 }
 
-// CLS_NO_SPLIT=1 (A/B experiments): every read is finished by the warp / CTA that built its histogram.
-static bool split_disabled() {
-    static const bool off = getenv("CLS_NO_SPLIT") != nullptr;
-    return off;
-}
 static inline ScanOut no_scan_out() {
     ScanOut so{};
     so.pairs = nullptr; so.meta = nullptr; so.cap = 0; so.counters = nullptr; so.ov_list = nullptr;
@@ -1469,37 +1461,37 @@ static inline ScanOut carve_scratch(void *scratch, uint32_t n_reads, uint32_t ca
     so.ov_list = so.counters + 16;
     return so;
 }
-template <int MAXSLOTS>
-static cudaError_t launch_descend(const DeviceIndex &ix, const PlaceParams &pp, const ScanOut &so, uint32_t first_read,
-                                  uint32_t n_reads, ResultRec *results, uint32_t fan_cap, int sm_count, cudaStream_t stream) {
-    // persistent CTAs: exactly as many as are resident at once (a larger grid would run a second, mostly empty wave)
+// The descent kernels run persistent CTAs: exactly as many as are resident at once (a larger grid would run a second,
+// mostly empty wave).  descend16_kernel after the short-read scan (at most kPairCap pairs per read) ...
+static cudaError_t launch_descend16(const DeviceIndex &ix, const PlaceParams &pp, const ScanOut &so, uint32_t first_read,
+                                    uint32_t n_reads, ResultRec *results, uint32_t fan_cap, int sm_count, cudaStream_t stream) {
     const size_t dsmem = (size_t)2 * fan_cap * 4 * 8;
     int occ = 0;
-    cudaError_t e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, descend_kernel<MAXSLOTS>, 256, dsmem);
+    cudaError_t e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, descend16_kernel, 256, dsmem);
+    if (e != cudaSuccess) return e;
+    if (occ < 1) occ = 1;
+    const uint32_t dgrid = std::min<uint32_t>((uint32_t)(sm_count * occ), (n_reads + 127) / 128);
+    descend16_kernel<<<dgrid, 256, dsmem, stream>>>(ix, pp, so, first_read, n_reads, results, fan_cap);
+    return cudaGetLastError();
+}
+// ... and descend_kernel<8> after the kb-scale scan (at most kPairCapWide pairs per read)
+static cudaError_t launch_descend8(const DeviceIndex &ix, const PlaceParams &pp, const ScanOut &so, uint32_t first_read,
+                                   uint32_t n_reads, ResultRec *results, uint32_t fan_cap, int sm_count, cudaStream_t stream) {
+    const size_t dsmem = (size_t)2 * fan_cap * 4 * 8;
+    int occ = 0;
+    cudaError_t e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, descend_kernel<8>, 256, dsmem);
     if (e != cudaSuccess) return e;
     if (occ < 1) occ = 1;
     uint32_t dgrid = (uint32_t)(sm_count * occ);
     const uint32_t need = (n_reads + 7) / 8;
     if (dgrid > need) dgrid = need;
-    static const bool groups = [] { const char *v = getenv("CLS_DESCEND_GROUPS"); return v ? atoi(v) != 0 : CLS_DESCEND_GROUPS != 0; }();
-    if (MAXSLOTS == 2 && groups) {
-        if ((e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, descend16_kernel, 256, dsmem)) != cudaSuccess) return e;
-        if (occ < 1) occ = 1;
-        dgrid = std::min<uint32_t>((uint32_t)(sm_count * occ), (n_reads + 127) / 128);
-        descend16_kernel<<<dgrid, 256, dsmem, stream>>>(ix, pp, so, first_read, n_reads, results, fan_cap);
-    } else {
-        descend_kernel<MAXSLOTS><<<dgrid, 256, dsmem, stream>>>(ix, pp, so, first_read, n_reads, results, fan_cap);
-    }
+    descend_kernel<8><<<dgrid, 256, dsmem, stream>>>(ix, pp, so, first_read, n_reads, results, fan_cap);
     return cudaGetLastError();
 }
 
 // ---- kb-scale reads, k = 35, closed models: scanfrag_kernel hashes and probes (frag_kernels.cuh), the placement kernel takes
 //      it from there.  The hits of one WAVE of reads live behind the hand-over scratch: 8 bytes per window and strand.
 constexpr size_t kFragWaveBytes = (size_t)1 << 30;
-static bool frag_disabled() {
-    static const bool off = getenv("CLS_NO_FRAG") != nullptr;
-    return off;
-}
 static inline uint32_t frag_hit_stride(const PlaceGeom &g) { return 2u * (g.max_len - 34u); }
 static inline uint32_t frag_wave_reads(uint32_t n_reads, const PlaceGeom &g) {
     const size_t per = (size_t)frag_hit_stride(g) * 8 + 1;
@@ -1520,8 +1512,7 @@ static cudaError_t launch_place_t(const DeviceIndex &ix, const PlaceParams &pp, 
     size_t smem;
     if (CTA) {
         // the tables of a kb-scale read leave room for two CTAs per SM: sixteen warps each keep the SM busy
-        static const int cta_warps = [] { const char *e = getenv("CLS_CTA_WARPS"); return e ? atoi(e) : 16; }();
-        warps = cta_warps;
+        warps = 16;
         if (group + ring * warps > 113 * 1024) warps = 8;
         smem = group + ring * warps;
     } else {
@@ -1543,7 +1534,7 @@ static cudaError_t launch_place_t(const DeviceIndex &ix, const PlaceParams &pp, 
     if (grid == 0) return cudaSuccess;
     // kb-scale reads of closed models: the histogram goes to the wide descent kernel when the caller gave scratch
     const bool split = CTA && CLOSED && scratch && scratch_bytes >= scratch_bytes_for(n_reads, kPairCapWide) &&
-                       (size_t)2 * g.fan_cap * 4 * 8 <= 48 * 1024 && !split_disabled();
+                       (size_t)2 * g.fan_cap * 4 * 8 <= 48 * 1024;
     ScanOut so = no_scan_out();
     if (split) {
         so = carve_scratch(scratch, n_reads, kPairCapWide);
@@ -1552,7 +1543,7 @@ static cudaError_t launch_place_t(const DeviceIndex &ix, const PlaceParams &pp, 
     bool two_phase = false;
     if constexpr (K == 35 && CLOSED && CTA) {
         const size_t pair_b = (scratch_bytes_for(n_reads, kPairCapWide) + 255) & ~(size_t)255;
-        two_phase = split && !frag_disabled() && !trace.rows && scratch_bytes >= pair_b + frag_scratch_bytes(n_reads, g);
+        two_phase = split && !trace.rows && scratch_bytes >= pair_b + frag_scratch_bytes(n_reads, g);
         if (two_phase) {
             char *base = reinterpret_cast<char *>(((uintptr_t)scratch + 255) & ~(uintptr_t)255) + pair_b;
             const uint32_t wave = frag_wave_reads(n_reads, g), stride = frag_hit_stride(g);
@@ -1602,7 +1593,7 @@ static cudaError_t launch_place_t(const DeviceIndex &ix, const PlaceParams &pp, 
         if (n_launches) ++*n_launches;
     }
     if (split) {
-        if ((e = launch_descend<8>(ix, pp, so, first_read, n_reads, results, g.fan_cap, sm_count, stream)) != cudaSuccess) return e;
+        if ((e = launch_descend8(ix, pp, so, first_read, n_reads, results, g.fan_cap, sm_count, stream)) != cudaSuccess) return e;
         if (n_launches) ++*n_launches;
     }
     return cudaSuccess;
@@ -1658,10 +1649,9 @@ size_t place_scratch_bytes(uint32_t n_reads, uint32_t max_len, uint32_t k, uint3
     if (max_len < k || n_reads == 0) return 0;
     const PlaceGeom g = make_place_geom(max_len, k, max_fanout);
     if (needs_giant(g)) return giant_scratch_bytes(n_reads, g);
-    if (split_disabled()) return 0;
     if (g.cta_per_read) {
         const size_t pair_b = (scratch_bytes_for(n_reads, kPairCapWide) + 255) & ~(size_t)255;
-        return k == 35 && !frag_disabled() ? pair_b + frag_scratch_bytes(n_reads, g) : pair_b;
+        return k == 35 ? pair_b + frag_scratch_bytes(n_reads, g) : pair_b;
     }
     return k == 35 ? scratch_bytes_for(n_reads, kPairCap) : 0;
 }
@@ -1716,22 +1706,20 @@ static cudaError_t launch_scan_t(const DeviceIndex &ix, const PlaceParams &pp, c
                                  const ReadDesc *reads, uint32_t first_read, uint32_t n_reads, ResultRec *results,
                                  const PlaceGeom &g, int sm_count, cudaStream_t stream, void *scratch, size_t scratch_bytes,
                                  uint32_t *n_launches) {
-    const bool split = CLOSED && scratch && scratch_bytes >= scratch_bytes_for(n_reads, kPairCap) && !split_disabled() &&
+    const bool split = CLOSED && scratch && scratch_bytes >= scratch_bytes_for(n_reads, kPairCap) &&
                        (size_t)2 * g.fan_cap * 4 * 8 <= 48 * 1024 && g.max_len <= Scan2Layout<8>::kMaxLen;
     if (!split) return launch_scan_old<CLOSED>(ix, pp, packed, reads, first_read, n_reads, results, g, sm_count, stream, nullptr, nullptr, n_launches);
     const ScanOut so = carve_scratch(scratch, n_reads, kPairCap);
     cudaError_t e = cudaMemsetAsync(so.counters, 0, 64, stream);
     if (e != cudaSuccess) return e;
     // a table well inside the 126 MB L2 wants registers, one that lives in HBM wants warps (scan2_kernels.cuh)
-    static const int force_minb = [] { const char *v = getenv("CLS_SCAN2_MINB"); return v ? atoi(v) : 0; }();
     const bool l2_resident = (ix.bucket_mask + 1) * sizeof(Slot) * 2 <= ((size_t)96 << 20);
-    const bool minb4 = force_minb ? force_minb == 4 : l2_resident;
     if (g.max_len > Scan2Layout<4>::kMaxLen) e = launch_scan2<8, 4>(ix, packed, reads, first_read, n_reads, so, sm_count, stream);
-    else if (minb4) e = launch_scan2<4, 4>(ix, packed, reads, first_read, n_reads, so, sm_count, stream);
+    else if (l2_resident) e = launch_scan2<4, 4>(ix, packed, reads, first_read, n_reads, so, sm_count, stream);
     else e = launch_scan2<4, 5>(ix, packed, reads, first_read, n_reads, so, sm_count, stream);
     if (e != cudaSuccess) return e;
     if (n_launches) ++*n_launches;
-    if ((e = launch_descend<2>(ix, pp, so, first_read, n_reads, results, g.fan_cap, sm_count, stream)) != cudaSuccess) return e;
+    if ((e = launch_descend16(ix, pp, so, first_read, n_reads, results, g.fan_cap, sm_count, stream)) != cudaSuccess) return e;
     if (n_launches) ++*n_launches;
     return launch_scan_old<true>(ix, pp, packed, reads, first_read, n_reads, results, g, sm_count, stream, so.ov_list, so.counters + 2, n_launches);
 }

@@ -51,33 +51,10 @@ __device__ __forceinline__ uint64_t mul5add(uint64_t x, uint32_t c) {
     return pack64((uint32_t)r, (uint32_t)(r >> 32) + hi * 5u);
 }
 
-// CLS_MUR_FMA (A/B): the placement kernels are bound by the ALU pipe (shifts, logic, adds: 77 % busy against 49 % of the
-// integer-multiply pipe, profiles/r2c); with it the shift of k ^= k >> 33 and the low halves of the 64-bit adds of the
-// finaliser go through IMAD instead.
-#ifndef CLS_MUR_FMA
-#define CLS_MUR_FMA 0
-#endif
+// k ^ (k >> 33)
 __device__ __forceinline__ uint64_t xorshift33(uint64_t k) {
     const uint32_t hi = (uint32_t)(k >> 32);
-#if CLS_MUR_FMA
-    uint32_t sh;
-    asm("mul.hi.u32 %0, %1, 0x80000000;" : "=r"(sh) : "r"(hi));   // hi >> 1
-    return pack64((uint32_t)k ^ sh, hi);
-#else
     return pack64((uint32_t)k ^ (hi >> 1), hi);
-#endif
-}
-
-__device__ __forceinline__ uint64_t add64(uint64_t a, uint64_t b) {
-#if CLS_MUR_FMA
-    uint64_t r;
-    asm("mad.wide.u32 %0, %1, 1, %2;" : "=l"(r) : "r"((uint32_t)a), "l"(b));   // b + a.lo, carry included
-    uint32_t rh;
-    asm("mad.lo.u32 %0, %1, 1, %2;" : "=r"(rh) : "r"((uint32_t)(a >> 32)), "r"((uint32_t)(r >> 32)));
-    return pack64((uint32_t)r, rh);
-#else
-    return a + b;
-#endif
 }
 
 __device__ __forceinline__ uint64_t fmix64_d(uint64_t k) {
@@ -101,9 +78,9 @@ __device__ __forceinline__ void mm_block(uint64_t &h1, uint64_t &h2, uint64_t k1
 
 __device__ __forceinline__ uint64_t mm_finish(uint64_t h1, uint64_t h2, uint64_t len) {
     h1 ^= len; h2 ^= len;
-    h1 = add64(h1, h2); h2 = add64(h2, h1);
+    h1 += h2; h2 += h1;
     h1 = fmix64_d(h1); h2 = fmix64_d(h2);
-    return add64(h1, h2);
+    return h1 + h2;
 }
 
 // Runtime-k variant (any k >= 1): byte-wise reads from a shared-memory ASCII string; used for k != 35.

@@ -355,7 +355,7 @@ cudaError_t launch_place_routed(const DeviceIndex &ix, const PlaceParams &pp, co
     const uint32_t need = (n_reads + warps - 1) / warps;
     if (grid > need) grid = need;
     const ProbeReply *rp = reinterpret_cast<const ProbeReply *>(replies);
-    const bool split = ix.closed && scratch && scratch_bytes >= scratch_bytes_for(n_reads, kPairCap) && !split_disabled() &&
+    const bool split = ix.closed && scratch && scratch_bytes >= scratch_bytes_for(n_reads, kPairCap) &&
                        (size_t)2 * g.fan_cap * 4 * 8 <= 48 * 1024;
     ScanOut so = no_scan_out();
     if (split) {
@@ -366,6 +366,6 @@ cudaError_t launch_place_routed(const DeviceIndex &ix, const PlaceParams &pp, co
     if ((e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, 226 * 1024)) != cudaSuccess) return e;
     kern<<<grid, warps * 32, smem, stream>>>(ix, pp, packed, reads, first_read, n_reads, results, g, n_shards, seg_cap, runs, slot_win, rp, so);
     if ((e = cudaGetLastError()) != cudaSuccess) return e;
-    if (split) e = launch_descend<2>(ix, pp, so, first_read, n_reads, results, g.fan_cap, sm_count, stream);
+    if (split) e = launch_descend16(ix, pp, so, first_read, n_reads, results, g.fan_cap, sm_count, stream);
     return e;
 }

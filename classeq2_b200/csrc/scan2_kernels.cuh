@@ -65,12 +65,9 @@ __device__ __forceinline__ void ld_bucket_if(bool p, uint64_t table, uint32_t bu
 constexpr uint32_t kListCap = 128;     // list area in entries
 constexpr uint32_t kListUse = 128;     // {node-set record, count} entries a read may append before the merge
 constexpr uint32_t kMergeSlots = 128;  // slots of the merge table (> kListUse: probing always terminates)
-#ifndef CLS_S2_BLOCK
-#define CLS_S2_BLOCK 2
-#endif
 // reads a warp takes from the global counter at a time: small, so that the last block of a launch is a small share of
 // a warp's work even in the chunked launches of cls_place_batch (about 30 reads per warp)
-constexpr uint32_t kScanBlock = CLS_S2_BLOCK;
+constexpr uint32_t kScanBlock = 2;
 
 // Per-warp shared memory, byte offsets from the warp's base (a multiple of 512: the ring halves alternate by
 // an XOR with 256 on the address).  PPS = passes per strand the geometry allows: 4 (reads of up to 162 bases)
@@ -107,18 +104,6 @@ __device__ __forceinline__ void premix_ring(uint32_t src, uint32_t sh8, uint32_t
 
 __device__ __forceinline__ void ld_bucket_if(bool p, uint64_t table, uint32_t bucket, uint64_t &h0, uint64_t &m0, uint64_t &h1,
                                              uint64_t &m1) {
-#if CLS_S2_LD128
-    asm volatile("{\n\t"
-                 ".reg .pred p;\n\t"
-                 ".reg .u64 a;\n\t"
-                 "setp.ne.u32 p, %6, 0;\n\t"
-                 "mad.wide.u32 a, %5, 32, %4;\n\t"
-                 "@p ld.global.nc.L1::no_allocate.v2.u64 {%0,%1}, [a];\n\t"
-                 "@p ld.global.nc.L1::no_allocate.v2.u64 {%2,%3}, [a+16];\n\t"
-                 "}"
-                 : "+l"(h0), "+l"(m0), "+l"(h1), "+l"(m1)
-                 : "l"(table), "r"(bucket), "r"((uint32_t)p));
-#else
     asm volatile("{\n\t"
                  ".reg .pred p;\n\t"
                  ".reg .u64 a;\n\t"
@@ -128,7 +113,6 @@ __device__ __forceinline__ void ld_bucket_if(bool p, uint64_t table, uint32_t bu
                  "}"
                  : "+l"(h0), "+l"(m0), "+l"(h1), "+l"(m1)
                  : "l"(table), "r"(bucket), "r"((uint32_t)p));
-#endif
 }
 
 // 16 two-bit codes -> 16 ASCII letters (four words), by spreading the codes into nibbles for PRMT on "ACTG"
@@ -166,26 +150,6 @@ __device__ __forceinline__ void decode_read16(const uint32_t *__restrict__ packe
         asm volatile("st.shared.v4.u32 [%0], {%1, %2, %3, %4};" ::"r"(sbase), "r"(q[0]), "r"(q[1]), "r"(q[2]), "r"(q[3]) : "memory");
     sts_u32(wb + (lane >= 16 ? Ly::oPkR : Ly::oPkF) + 4u * t, v);
 }
-
-// A/B switches of this file (tools/build_variants.sh); the defaults are what measured best
-#ifndef CLS_S2_DIRECT
-#define CLS_S2_DIRECT 1       // lists of up to 32 entries are merged in registers (one match.any), not through the table
-#endif
-#ifndef CLS_S2_FASTDECODE
-#define CLS_S2_FASTDECODE 1   // decode_read16 for the PPS = 4 geometry
-#endif
-#ifndef CLS_S2_PREFETCH
-#define CLS_S2_PREFETCH 1     // L1 prefetch of the next read's packed bases
-#endif
-#ifndef CLS_S2_PREDLOAD
-#define CLS_S2_PREDLOAD 1     // lanes without a window do not load a bucket (0: they load bucket 0)
-#endif
-#ifndef CLS_S2_BLOOM
-#define CLS_S2_BLOOM 1        // a miss follows the overflow chain only if the home bucket's 8-bit filter has its bit
-#endif
-#ifndef CLS_S2_LD128
-#define CLS_S2_LD128 0        // the bucket as two 128-bit loads instead of one 256-bit load
-#endif
 
 // One pass (32 windows) whose bucket load is in flight.
 struct Flight {
@@ -247,12 +211,8 @@ __device__ __forceinline__ void scan2_consume(Scan2Ctx &cx, const DeviceIndex &i
     // free slots carry a hash that no probe of their bucket can ask for (index_build.cpp), so equality is a hit
     bool e0 = f.q0 == f.h, e1 = f.q1 == f.h;
     // rare: the bucket overflowed at build time and the hash is not in it - follow the chain (all lanes stay together)
-#if CLS_S2_BLOOM
     // ... and the home bucket's filter (index_build.cpp: one of eight bits per entry that went elsewhere) has its bit
     bool chase = valid && !(e0 || e1) && (((uint32_t)(f.qm1 >> 32) >> (kBloomShift + (((uint32_t)(f.h >> 32) >> 8) & 7u))) & 1u);
-#else
-    bool chase = valid && !(e0 || e1) && ((uint32_t)(f.qm0 >> 32) & kOverflowBit);
-#endif
     while (__any_sync(kFull, chase)) {
         if (chase) {
             b = (b + 1) & cx.bmask;
@@ -317,11 +277,7 @@ __device__ __forceinline__ void scan2_step(Scan2Ctx &cx, const DeviceIndex &ix, 
     if (it > 0 && it <= cx.n_total) scan2_consume<PPS>(cx, ix, wm, it - 1u, prev);
     if (more) {
         const bool valid = (int32_t)(threadIdx.x & 31u) < cur.lim;
-#if CLS_S2_PREDLOAD
         ld_bucket_if(valid, cx.table, (uint32_t)cur.h & cx.bmask, cur.q0, cur.qm0, cur.q1, cur.qm1);
-#else
-        ld_bucket_if(true, cx.table, valid ? (uint32_t)cur.h & cx.bmask : 0u, cur.q0, cur.qm0, cur.q1, cur.qm1);
-#endif
     }
 }
 
@@ -377,16 +333,14 @@ __global__ void __launch_bounds__(256, MINB)
         // warp-uniform loads: the loop bounds derived from the descriptor live in uniform registers
         const ReadDesc rd = reads[first_read + r];
         const uint32_t L = rd.len;
-#if CLS_S2_PREFETCH
         if (blk_used < kScanBlock && r + 1u < n_reads) {   // the next read's packed bases, while this one is placed
             const uint32_t nxt = reads[first_read + r + 1u].word_off;
             if (lane < 3) asm volatile("prefetch.global.L1 [%0];" ::"l"(reinterpret_cast<const char *>(packed + nxt) + 32u * lane));
         }
-#endif
         cx.W = L - 34u;  // host guarantees 35 <= L <= Ly::kMaxLen
         sts_v4(cx.wb + Ly::oFilter + 16u * lane, 0u);
         sts_v4(cx.wb + Ly::oFilter + 512u + 16u * lane, 0u);
-        if constexpr (PPS == 4 && CLS_S2_FASTDECODE) decode_read16<PPS>(packed + rd.word_off, L, cx.wb);
+        if constexpr (PPS == 4) decode_read16<PPS>(packed + rd.word_off, L, cx.wb);
         else decode_read(packed + rd.word_off, L, wm, Ly::kPkWords);
         cx.n_chunks = (cx.W + 31u) >> 5; cx.n_total = 2u * cx.n_chunks;
         cx.n_list = 0; cx.gate_next = 0;
@@ -407,7 +361,7 @@ __global__ void __launch_bounds__(256, MINB)
         bool overflow = cx.n_list > kListUse;
         uint32_t D = 0, n_matched = 0;
         uint2 *row = so.pairs + (size_t)r * so.cap;
-        if (CLS_S2_DIRECT && cx.n_list <= 32) {
+        if (cx.n_list <= 32) {
             // one entry per lane: entries of the same node-set record are summed into the lowest lane that holds it (the
             // descent kernel runs several reads side by side when they have few node sets, so fewer pairs pay)
             const bool valid = lane < cx.n_list;

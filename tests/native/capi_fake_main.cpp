@@ -78,8 +78,7 @@ static void compare(const Batch &b, Results &got, const void *orc, const cls_par
     g_reads += (long)n;
 }
 
-int main(int argc, char **argv) {
-    const bool threads_only = argc > 1 && !strcmp(argv[1], "threads");   // the ThreadSanitizer build: the scenarios with more than one host thread
+int main() {
     const int scale = 1;
     setenv("CLS_CHUNK_MBASES", "1", 1);           // 1 Mi bases per chunk: a few thousand reads are already several chunks
     setenv("CLS_HOST_THREADS", "4", 0);   // (not overwritten: a run with one thread takes the pool out)
@@ -156,7 +155,6 @@ int main(int argc, char **argv) {
     // (a chunk holds at least 4 096 reads: 9 000 reads are several chunks, 1 500 one)
     for (int mode = 1; mode <= 3; ++mode)
         for (int pin = 0; pin < 2; ++pin) {
-            if (threads_only && !(mode == 2 && pin == 0)) continue;
             const Batch shorts = make_reads((mode == 2 && pin == 0) || (mode == 3 && pin == 1) ? 9000 : 1500, 36, 90, 0);   // (host packing over several chunks: scenario 2)
             void *pinned = nullptr;
             cudaHostAlloc(&pinned, shorts.bases.size(), cudaHostAllocDefault);
@@ -174,7 +172,6 @@ int main(int argc, char **argv) {
             cudaFreeHost(pinned);
         }
     EXPECT(fakek::pack_launches > 0);
-    if (!threads_only) {
     // ---- 2. late in a batch of short reads: one read that is too short / too long (the just-in-time plan falls back to the
     //      general one), or reads with an invalid base (it does not: the packer that meets them flags them) ------
     for (int kind_of = 0; kind_of < 3; ++kind_of)
@@ -325,10 +322,9 @@ int main(int argc, char **argv) {
         cls_fasta_records dr{};
         EXPECT(cls_fasta_upload(ix, reinterpret_cast<const uint8_t *>(text.data()), text.size(), &rb, &dr) == CLS_ERR_UNSUPPORTED && !rb);
     }
-    }
     // ---- 5c. the whole use-case in one call: cls_place_sequences = reader + the REAL cls_place_batch per batch of 3 000 queries
     //      + the writer, which renders and appends batch i on a second thread while batch i + 1 is placed ------------------------------
-    if (threads_only || fakecuda::async()) {                  // (a scenario about threads: the runs with asynchronous streams take it)
+    if (fakecuda::async()) {                  // (a scenario about threads: the runs with asynchronous streams take it)
         STEP("5c. cls_place_sequences");
         const uint64_t nn = node_id.size();
         std::vector<int64_t> parent_id(nn, -1);
@@ -438,7 +434,7 @@ int main(int argc, char **argv) {
     }
     // ---- 8. an allocation that fails (device or pinned), at every position in turn: the call reports it, nothing is leaked,
     //      and the same handle places the batch once memory is back -----------------------------------------------------------------
-    if (!threads_only && !fakecuda::async()) {
+    if (!fakecuda::async()) {
         STEP("8. failing allocations");
         const Batch b = make_reads(40, 30, 300, 7);
         const cls_batch bv = b.view();
@@ -558,5 +554,5 @@ int main(int argc, char **argv) {
     EXPECT(fakecuda::live_allocs() == 0);                                                // every device / pinned buffer was released
     printf("bad=%ld reads=%ld place_launches=%llu pack_launches=%llu\n", g_bad, g_reads, (unsigned long long)fakek::place_launches.load(),
            (unsigned long long)fakek::pack_launches.load());
-    return g_bad == 0 && g_reads > (threads_only ? 15000 : 50000) ? 0 : 1;
+    return g_bad == 0 && g_reads > 50000 ? 0 : 1;
 }

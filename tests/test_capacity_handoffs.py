@@ -4,8 +4,8 @@ Most branches of these paths are taken only when a read outgrows a fixed table:
   * gather_kernel (frag_kernels.cuh): up to kPairCapWide = 256 distinct node-set records go to descend_kernel<8>, up to
     kGListCap = 1024 to descend_wide_kernel, more (or D + 1 > 2(L - 34), or more than kGSetSlots = 1024 distinct table
     slots behind collided filter bits) back to place_kernel<35, true, true>;
-  * the short-read path: the four- and two-per-warp groups of descend16_kernel, descend_kernel<2>, and the kPairCap = 64
-    overflow into scan_kernel;
+  * the short-read path: the four- and two-per-warp groups of descend16_kernel, its one-read-per-warp walk, and the
+    kPairCap = 64 overflow into scan_kernel;
   * launch_place_t / launch_giant (kernels.cu): second and later scratch waves.
 Real models make reads that reach them rare, so the models here are built to a given number of records per read:
 a tree with multifurcations, a pool of upward-closed node sets per template read, and hit i of template t filed under
@@ -352,8 +352,8 @@ def test_gather_exact_set_overflow(cq):
 # ---- 4. short-read hand-off boundaries ----------------------------------------------------------------------------------
 @gpu
 def test_short_read_record_count_boundaries(cq):
-    """150-base reads with D around the groups of descend16_kernel (8, 16), descend_kernel<2> (32) and the kPairCap = 64
-    overflow into scan_kernel, interleaved so that groups mix record counts; also through the routed pipeline."""
+    """150-base reads with D around the groups of descend16_kernel (8, 16), its one-read-per-warp walk (32 records per
+    register slot) and the kPairCap = 64 overflow into scan_kernel, interleaved so that groups mix record counts; also through the routed pipeline."""
     rng = np.random.default_rng(4)
     Ds = (1, 8, 9, 16, 17, 32, 33, 64, 65)
     spec = [(150, D, 0.3 if D >= 32 and j == 1 else 0.0) for D in Ds for j in range(4)]

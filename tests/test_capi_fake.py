@@ -67,10 +67,7 @@ def runs(tmp_path_factory):
     # missing dependency between streams, or between a stream and the host, is a data race there
     procs = {"asan": subprocess.Popen([exes["asan"]], stdout=subprocess.PIPE, stderr=subprocess.PIPE, text=True),
              "tsan": subprocess.Popen([exes["tsan"]], stdout=subprocess.PIPE, stderr=subprocess.PIPE, text=True,
-                                      env=dict(os.environ, FAKE_CUDA_ASYNC="1")),
-             # the two-stream pipeline (CLS_PIPE=2, an A/B knob): the scenarios with several host threads
-             "tsan_pipe2": subprocess.Popen([exes["tsan"], "threads"], stdout=subprocess.PIPE, stderr=subprocess.PIPE, text=True,
-                                            env=dict(os.environ, FAKE_CUDA_ASYNC="1", CLS_PIPE="2"))}
+                                      env=dict(os.environ, FAKE_CUDA_ASYNC="1"))}
     out = {}
     for name, p in procs.items():
         try:
@@ -92,13 +89,10 @@ def test_place_batch_host_side_equals_the_oracle_under_asan(runs):
 def test_place_batch_streams_and_threads_are_race_free_under_tsan(runs):
     """Every scenario again with the streams of the fake runtime as worker threads: copies, fake kernels and event waits run
     in stream order next to the host thread, so the dependencies of the three-stream pipeline (copies in -> kernels ->
-    copies out, the staging ring, the scratch buffers, the scatter of finished chunks) are what keeps this free of races.
-    Dropping the kernel stream's wait for the copy-in of the later chunks is reported here (checked by mutation), and this
-    is how the one real finding came up: with device packing the two-stream pipeline (CLS_PIPE=2) let a chunk's pack kernel
-    read bases that the other stream was still copying - device packing now always takes the three-stream pipeline."""
-    for name in ("tsan", "tsan_pipe2"):
-        r = runs[name]
-        if "FATAL: ThreadSanitizer" in r.stderr and "unexpected memory mapping" in r.stderr:
-            pytest.skip("ThreadSanitizer cannot map its shadow memory in this container")
-        assert "WARNING: ThreadSanitizer" not in r.stderr and "[timed out]" not in r.stderr, (name, r.stderr[:4000])
-        assert r.returncode == 0 and r.stdout.startswith("bad=0 "), (name, r.returncode, r.stdout, r.stderr[-1500:])
+    copies out, the staging ring, the scratch buffer, the scatter of finished chunks) are what keeps this free of races.
+    Dropping the kernel stream's wait for the copy-in of the later chunks is reported here (checked by mutation)."""
+    r = runs["tsan"]
+    if "FATAL: ThreadSanitizer" in r.stderr and "unexpected memory mapping" in r.stderr:
+        pytest.skip("ThreadSanitizer cannot map its shadow memory in this container")
+    assert "WARNING: ThreadSanitizer" not in r.stderr and "[timed out]" not in r.stderr, r.stderr[:4000]
+    assert r.returncode == 0 and r.stdout.startswith("bad=0 "), (r.returncode, r.stdout, r.stderr[-1500:])

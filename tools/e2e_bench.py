@@ -1,7 +1,7 @@
 #!/usr/bin/env python
-"""End-to-end timing of cls_place_batch (host ASCII buffers in, host result arrays out) on config 2's workload, for A/B of
-the host-side pipeline knobs: CLS_PIPE=3 (three streams chained by events), CLS_CHUNK_MBASES, CLS_CHUNK_RAMP,
-CLS_HOST_THREADS; CLASSEQ_B200_LIB picks a kernel variant.  usage: [ENV=...] python tools/e2e_bench.py [n_reads=1000000]"""
+"""End-to-end timing of cls_place_batch (host ASCII buffers in, host result arrays out) on config 2's workload, under the
+host-side knobs CLS_CHUNK_MBASES, CLS_HOST_THREADS and CLS_PACK; CLASSEQ_B200_LIB picks the library.
+usage: [ENV=...] python tools/e2e_bench.py [n_reads=1000000]"""
 import os
 import sys
 import time
@@ -33,7 +33,7 @@ for _ in range(10):
     ix.place_batch_into(bases, offsets, out)
     ts.append(time.perf_counter() - t0)
 dt = float(np.mean(ts))
-knobs = {k: os.environ[k] for k in ("CLS_PIPE", "CLS_CHUNK_MBASES", "CLS_CHUNK_RAMP", "CLS_HOST_THREADS", "CLASSEQ_B200_LIB", "CLS_PACK", "PIN") if k in os.environ}
+knobs = {k: os.environ[k] for k in ("CLS_CHUNK_MBASES", "CLS_HOST_THREADS", "CLASSEQ_B200_LIB", "CLS_PACK", "PIN") if k in os.environ}
 print(f"config{cfg} n={n} replicas={n_dev} {knobs} e2e {dt * 1e3:.2f} ms (min {min(ts) * 1e3:.2f})  {n / dt / 1e6:.1f} M reads/s  "
       f"status_hist={np.bincount(out.status, minlength=11).tolist()} sum(node)={int(out.node_id.sum())}",
       {k: round(v, 2) for k, v in ix.timing().items()})
