@@ -21,6 +21,8 @@ CLS_ERR_UNSUPPORTED = -3
 CLS_ERR_OUT_OF_MEMORY = -4
 CLS_ERR_NCCL = -5
 
+QUERY_FASTQ = 0x100   # CLS_QUERY_FASTQ: ORed into the format of cls_sequences_open / cls_place_sequences
+
 KIND_ROOT, KIND_NODE, KIND_LEAF = 0, 1, 2
 MODEL_ROOT_CHILDREN_NONE = 1
 MODEL_FORCE_GENERAL_SETS = 2
@@ -123,6 +125,7 @@ PROTOTYPES = {
     "cls_get_timing": (C.c_int, [C.c_void_p, C.POINTER(Timing)]),
     "cls_set_pack_mode": (C.c_int, [C.c_int]),
     "cls_fasta_upload": (C.c_int, [C.c_void_p, u8p, C.c_uint64, C.POINTER(C.c_void_p), C.POINTER(FastaRecords)]),
+    "cls_fastq_upload": (C.c_int, [C.c_void_p, u8p, C.c_uint64, C.POINTER(C.c_void_p), C.POINTER(FastaRecords)]),
     "cls_index_create_shard": (C.c_int, [C.POINTER(ModelView), C.c_int, C.c_uint32, C.c_uint32, C.POINTER(C.c_void_p)]),
     "cls_index_create_multi": (C.c_int, [C.POINTER(ModelView), C.c_uint64, C.POINTER(C.c_void_p)]),
     "cls_index_create_devices": (C.c_int, [C.POINTER(ModelView), C.c_uint32, C.POINTER(C.c_int), C.POINTER(C.c_void_p)]),
@@ -145,6 +148,7 @@ PROTOTYPES = {
     "cls_text_free": (None, [C.c_void_p]),
     "cls_fasta_read": (C.c_int, [u8p, C.c_uint64, C.POINTER(C.c_void_p), C.POINTER(FastaHostRecords)]),
     "cls_fasta_text_destroy": (None, [C.c_void_p]),
+    "cls_fastq_read": (C.c_int, [u8p, C.c_uint64, C.POINTER(C.c_void_p), C.POINTER(FastaHostRecords)]),
     "cls_sequences_open": (C.c_int, [C.c_char_p, C.c_char_p, C.c_uint32, C.c_uint32, C.POINTER(C.c_void_p), C.POINTER(Batch)]),
     "cls_sequences_write": (C.c_int, [C.c_void_p, C.POINTER(RecordTree), C.c_uint64, C.POINTER(Result)]),
     "cls_sequences_close": (None, [C.c_void_p]),

@@ -1108,6 +1108,47 @@ int cls_batch_upload(cls_index *ix, const cls_batch *batch, cls_resident_batch *
     return CLS_OK;
 } CLS_ABI_CATCH
 
+// The tail of both text ingests: the records' lengths are in rb->fa_length and their first kept base in `src`; plan them
+// with the planner of cls_batch_upload and pack them from the compacted codes on the device.
+static int pack_ingested(cls_index *ix, cls_resident_batch *rb, const uint8_t *d_codes, const std::vector<uint64_t> &src, cudaStream_t st) {
+    const auto &ln = rb->fa_length;
+    const uint64_t n = ln.size();
+    std::vector<uint64_t> offsets(n + 1, 0);
+    for (uint64_t i = 0; i < n; ++i) offsets[i + 1] = offsets[i] + ln[i];
+    cls_batch fake{n, reinterpret_cast<const uint8_t *>(offsets.data()), offsets.data()};   // plan_batch never reads the bases
+    std::vector<uint32_t> word_off;
+    int rc = plan_batch(&fake, ix->dix.k_size, ix->dix.max_fanout, rb->lay, word_off);
+    if (rc != CLS_OK) return rc;
+    const PackedLayout &lay = rb->lay;
+    const size_t words_b = (size_t)lay.n_words * 4, descs_b = (size_t)lay.n_device * sizeof(ReadDesc), res_b = (size_t)lay.n_device * sizeof(ResultRec);
+    CU_TRY(rb->d_words.reserve(words_b + 16)); CU_TRY(rb->d_descs.reserve(descs_b + 16)); CU_TRY(rb->d_results.reserve(res_b + 32));
+    if (lay.n_device) {   // the pinned result buffer is allocated by the first cls_resident_fetch
+        DevBuf d_src, d_woff, d_len;
+        struct Free { std::vector<DevBuf *> b; ~Free() { for (auto *x : b) x->release(); } } guard{{&d_src, &d_woff, &d_len}};
+        std::vector<ReadDesc> descs(lay.n_device);
+        std::vector<uint64_t> src_dev(lay.n_device);
+        std::vector<uint32_t> len_dev(lay.n_device);
+        parallel_for(lay.n_device, 1 << 15, [&](uint64_t j0, uint64_t j1) {
+            for (uint64_t j = j0; j < j1; ++j) {
+                const uint32_t i = lay.perm[j];
+                descs[j] = ReadDesc{word_off[j], ln[i]};
+                src_dev[j] = src[i];
+                len_dev[j] = ln[i];
+            }
+        });
+        CU_TRY(d_src.reserve(src_dev.size() * 8)); CU_TRY(d_woff.reserve(word_off.size() * 4)); CU_TRY(d_len.reserve(len_dev.size() * 4));
+        CU_TRY(cudaMemcpyAsync(d_src.p, src_dev.data(), src_dev.size() * 8, cudaMemcpyHostToDevice, st));
+        CU_TRY(cudaMemcpyAsync(d_woff.p, word_off.data(), (size_t)lay.n_device * 4, cudaMemcpyHostToDevice, st));
+        CU_TRY(cudaMemcpyAsync(d_len.p, len_dev.data(), len_dev.size() * 4, cudaMemcpyHostToDevice, st));
+        CU_TRY(cudaMemcpyAsync(rb->d_descs.p, descs.data(), descs_b, cudaMemcpyHostToDevice, st));
+        CU_TRY(launch_fasta_pack(d_codes, (const uint64_t *)d_src.p, (const uint32_t *)d_woff.p, (const uint32_t *)d_len.p,
+                                 lay.n_device, (uint32_t *)rb->d_words.p, ix->sm_count, st));
+        CU_TRY(cudaMemsetAsync(rb->d_results.p, 0xFF, res_b, st));
+        CU_TRY(cudaStreamSynchronize(st));
+    }
+    return CLS_OK;
+}
+
 // ---- FASTA ingest on the device (SURVEY.md section 8f row 3; file_or_stdin.rs:76-116, sequence.rs:47-56) -----------
 int cls_fasta_upload(cls_index *ix, const uint8_t *text, uint64_t n_bytes, cls_resident_batch **out, cls_fasta_records *records) try {
     if (!ix || !out || !records || (n_bytes && !text)) return fail(CLS_ERR_INVALID_ARGUMENT, "NULL argument");
@@ -1123,9 +1164,9 @@ int cls_fasta_upload(cls_index *ix, const uint8_t *text, uint64_t n_bytes, cls_r
     auto rb = std::make_unique<cls_resident_batch>();
     rb->device = ix->device;
     cudaStream_t st = nullptr;
-    DevBuf d_text, d_tiles, d_bases, d_misc, d_codes, d_hpos, d_hkept, d_hflag, d_src, d_woff, d_len;
+    DevBuf d_text, d_tiles, d_bases, d_misc, d_codes, d_hpos, d_hkept, d_hflag;
     struct Free { std::vector<DevBuf *> b; ~Free() { for (auto *x : b) x->release(); } }
-        guard{{&d_text, &d_tiles, &d_bases, &d_misc, &d_codes, &d_hpos, &d_hkept, &d_hflag, &d_src, &d_woff, &d_len}};
+        guard{{&d_text, &d_tiles, &d_bases, &d_misc, &d_codes, &d_hpos, &d_hkept, &d_hflag}};
     const uint32_t nt = fasta_n_tiles(n_bytes);
     TileBase totals{0, 0, 0, 0};
     uint32_t non_ascii = 0;
@@ -1197,39 +1238,8 @@ int cls_fasta_upload(cls_index *ix, const uint8_t *text, uint64_t n_bytes, cls_r
         }
     });
     lap("header ends");
-    // ---- length classes, device order, packed layout: the same planner as cls_batch_upload ------------------------
-    std::vector<uint64_t> offsets(n + 1, 0);
-    for (uint64_t i = 0; i < n; ++i) offsets[i + 1] = offsets[i] + ln[i];
-    cls_batch fake{n, reinterpret_cast<const uint8_t *>(offsets.data()), offsets.data()};   // plan_batch never reads the bases
-    std::vector<uint32_t> word_off;
-    int rc = plan_batch(&fake, ix->dix.k_size, ix->dix.max_fanout, rb->lay, word_off);
+    const int rc = pack_ingested(ix, rb.get(), (const uint8_t *)d_codes.p, src, st);
     if (rc != CLS_OK) return rc;
-    lap("plan");
-    const PackedLayout &lay = rb->lay;
-    const size_t words_b = (size_t)lay.n_words * 4, descs_b = (size_t)lay.n_device * sizeof(ReadDesc), res_b = (size_t)lay.n_device * sizeof(ResultRec);
-    CU_TRY(rb->d_words.reserve(words_b + 16)); CU_TRY(rb->d_descs.reserve(descs_b + 16)); CU_TRY(rb->d_results.reserve(res_b + 32));
-    if (lay.n_device) {   // the pinned result buffer is allocated by the first cls_resident_fetch
-        std::vector<ReadDesc> descs(lay.n_device);
-        std::vector<uint64_t> src_dev(lay.n_device);
-        std::vector<uint32_t> len_dev(lay.n_device);
-        parallel_for(lay.n_device, 1 << 15, [&](uint64_t j0, uint64_t j1) {
-            for (uint64_t j = j0; j < j1; ++j) {
-                const uint32_t i = lay.perm[j];
-                descs[j] = ReadDesc{word_off[j], ln[i]};
-                src_dev[j] = src[i];
-                len_dev[j] = ln[i];
-            }
-        });
-        CU_TRY(d_src.reserve(src_dev.size() * 8)); CU_TRY(d_woff.reserve(word_off.size() * 4)); CU_TRY(d_len.reserve(len_dev.size() * 4));
-        CU_TRY(cudaMemcpyAsync(d_src.p, src_dev.data(), src_dev.size() * 8, cudaMemcpyHostToDevice, st));
-        CU_TRY(cudaMemcpyAsync(d_woff.p, word_off.data(), (size_t)lay.n_device * 4, cudaMemcpyHostToDevice, st));
-        CU_TRY(cudaMemcpyAsync(d_len.p, len_dev.data(), len_dev.size() * 4, cudaMemcpyHostToDevice, st));
-        CU_TRY(cudaMemcpyAsync(rb->d_descs.p, descs.data(), descs_b, cudaMemcpyHostToDevice, st));
-        CU_TRY(launch_fasta_pack((const uint8_t *)d_codes.p, (const uint64_t *)d_src.p, (const uint32_t *)d_woff.p, (const uint32_t *)d_len.p,
-                                 lay.n_device, (uint32_t *)rb->d_words.p, ix->sm_count, st));
-        CU_TRY(cudaMemsetAsync(rb->d_results.p, 0xFF, res_b, st));
-        CU_TRY(cudaStreamSynchronize(st));
-    }
     lap("pack");
     records->n_records = n;
     records->header_begin = hb.data();
@@ -1238,6 +1248,37 @@ int cls_fasta_upload(cls_index *ix, const uint8_t *text, uint64_t n_bytes, cls_r
     *out = rb.release();
     return CLS_OK;
 } CLS_ABI_CATCH
+
+// ---- for the FASTQ ingest (fastq_ingest.cpp): the handle a resident batch of `ix` lives on, and the batch built from the
+//      records a text ingest found (their first kept base `src` in the compacted codes on that device) -----------------------
+}  // extern "C"
+namespace cls {
+cls_index *ingest_home(cls_index *ix, int *device, int *sm_count) {
+    if (!ix->shards.empty()) ix = ix->shards[0].get();       // a sharded handle: resident batches live on its first shard's device
+    if (!ix->replicas.empty()) ix = ix->replicas[0].get();   // a multi-device handle: resident batches live on its first device
+    *device = ix->device;
+    *sm_count = ix->sm_count;
+    return ix;
+}
+
+int ingest_finish(cls_index *home, const uint8_t *d_codes, std::vector<uint64_t> &hb, std::vector<uint64_t> &he, std::vector<uint32_t> &ln,
+                  const std::vector<uint64_t> &src, cudaStream_t st, cls_resident_batch **out, cls_fasta_records *records) try {
+    auto rb = std::make_unique<cls_resident_batch>();
+    rb->device = home->device;
+    rb->fa_header_begin.swap(hb);
+    rb->fa_header_end.swap(he);
+    rb->fa_length.swap(ln);
+    const int rc = pack_ingested(home, rb.get(), d_codes, src, st);
+    if (rc != CLS_OK) return rc;
+    records->n_records = rb->fa_length.size();
+    records->header_begin = rb->fa_header_begin.data();
+    records->header_end = rb->fa_header_end.data();
+    records->length = rb->fa_length.data();
+    *out = rb.release();
+    return CLS_OK;
+} CLS_ABI_CATCH
+}  // namespace cls
+extern "C" {
 
 int cls_place_resident(cls_index *ix, cls_resident_batch *rb, const cls_params *params, void *stream) try {
     if (!ix || !rb || !params) return fail(CLS_ERR_INVALID_ARGUMENT, "NULL argument");

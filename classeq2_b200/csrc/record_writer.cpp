@@ -9,11 +9,13 @@
 //                        One block of records per task on the host pool, concatenated in input order.
 //   cls_filter_sequence  SequenceBody::remove_non_iupac_from_sequence (sequence.rs:47-56)
 //   cls_fasta_read       the reader of file_or_stdin.rs:76-116 (chunks of whole lines scanned on the host pool)
+//   cls_fastq_read       the FASTQ reader (four-line records; chunks of whole records read on the host pool)
 //   cls_sequences_open / cls_sequences_write / cls_place_sequences
 //                        the use-case itself (mod.rs:43-270): path handling, reader, cls_place_batch, writer
 // The Python mirror (classeq2_b200/placement.py) is the second implementation of all of it; tests hold the two
 // byte-identical, and both equal to a reference-written result file.
 #include <algorithm>
+#include <atomic>
 #include <charconv>
 #include <cstdio>
 #include <stdexcept>
@@ -31,6 +33,7 @@
 #include <sys/types.h>
 
 #include "../../include/classeq_b200.h"
+#include "fastq_rules.hpp"
 #include "host_pool.hpp"
 
 namespace cls {
@@ -837,6 +840,203 @@ extern "C" int cls_fasta_read(const uint8_t *text, uint64_t n_bytes, cls_fasta_t
 
 extern "C" void cls_fasta_text_destroy(cls_fasta_text *t) { delete t; }
 
+// ---- FASTQ queries (the rules are in include/classeq_b200.h, next to CLS_QUERY_FASTQ).  The reference has no FASTQ
+//      reader; these rules make a FASTQ file and its FASTA rendering place identically.  cls_fastq_upload applies the same
+//      rules on the device and reports its first bad record through the helpers below. -------------------------------------
+namespace cls {
+
+const char *fastq_reason(int code) {
+    switch (code) {
+    case kFastqBlankLine: return "blank line inside the records";
+    case kFastqNoAt: return "title line does not start with '@'";
+    case kFastqTruncated: return "truncated record (fewer than four lines)";
+    case kFastqNoPlus: return "separator line does not start with '+'";
+    case kFastqQualityLength: return "quality length differs from sequence length";
+    case kFastqTitleUtf8: return "title is not valid UTF-8";
+    default: return "malformed record";
+    }
+}
+
+int fastq_fail(uint64_t record, int code) {   // record: 0-based
+    return set_last_error(CLS_ERR_INVALID_ARGUMENT, "malformed FASTQ record " + std::to_string(record + 1) + ": " + fastq_reason(code));
+}
+
+// Records of the text: the records end at the last non-blank line (blank lines may only follow the last record).  A line
+// is blank when nothing but its terminator ("\n" or "\r\n") is in it.
+uint64_t fastq_n_records(const uint8_t *text, uint64_t n, uint64_t n_newlines) {
+    uint64_t e = n, blank = 0;
+    while (e > 0 && text[e - 1] == '\n') {
+        uint64_t s = e - 1;
+        if (s > 0 && text[s - 1] == '\r') --s;
+        if (s > 0 && text[s - 1] != '\n') break;   // the terminator of a line with content
+        e = s;
+        ++blank;
+    }
+    const uint64_t lines = n_newlines - blank + (e > 0 && text[e - 1] != '\n' ? 1 : 0);   // lines up to the last non-blank one
+    return lines ? (lines - 1) / 4 + 1 : 0;
+}
+
+// First record r < n_records whose title text[hb[r] .. he[r]) is not valid UTF-8, or n_records.
+uint64_t fastq_first_bad_title(const uint8_t *text, const uint64_t *hb, const uint64_t *he, uint64_t n_records) {
+    std::atomic<uint64_t> first{n_records};
+    parallel_for(n_records, 1 << 14, [&](uint64_t a, uint64_t b) {
+        for (uint64_t r = a; r < b && r < first.load(std::memory_order_relaxed); ++r) {
+            bool ascii = true;
+            for (uint64_t i = hb[r]; i < he[r] && ascii; ++i) ascii = text[i] < 0x80;
+            if (!ascii && !valid_utf8(text + hb[r], he[r] - hb[r])) {
+                uint64_t cur = first.load();
+                while (r < cur && !first.compare_exchange_weak(cur, r)) {}
+                break;
+            }
+        }
+    });
+    return first.load();
+}
+
+}  // namespace cls
+
+// cls_fastq_read: chunks of ~2 MiB cut at line ends; their newlines are counted side by side, which gives the line number
+// at every chunk start; each chunk is then moved forward to its first record start (a line number that is a multiple of
+// 4), so that every chunk holds whole records and is read without knowing anything about the others.  A wave of chunks
+// at a time is read on the host pool into buffers of their own, and appended in file order.
+namespace {
+
+struct FqLine {
+    uint64_t begin, end, next;   // content [begin, end) ("\n" / "\r\n" excluded); next: the first byte after the terminator
+};
+FqLine fq_line(const uint8_t *text, uint64_t n, uint64_t a) {
+    const uint8_t *nl = static_cast<const uint8_t *>(memchr(text + a, '\n', n - a));
+    if (!nl) return FqLine{a, n, n};
+    uint64_t e = (uint64_t)(nl - text);
+    const uint64_t next = e + 1;
+    if (e > a && text[e - 1] == '\r') --e;
+    return FqLine{a, e, next};
+}
+
+struct FqChunk {
+    uint64_t a = 0, b = 0;         // whole records [a, b) of the text
+    uint64_t first = 0;            // number of its first record
+    uint64_t lines = 0;            // (line counting) newlines in the raw chunk
+    std::vector<uint64_t> hb, he, len;
+    std::vector<uint8_t> bases;
+    uint64_t kept = 0;
+    uint64_t bad = ~0ull;          // first bad record, 0-based (~0: none)
+    int code = 0;
+};
+
+void fastq_read_chunk(const uint8_t *text, uint64_t n, uint64_t n_records, FqChunk &c) {
+    c.hb.clear(); c.he.clear(); c.len.clear();
+    c.kept = 0;
+    c.bad = ~0ull;
+    if (c.bases.size() < c.b - c.a) c.bases.resize(c.b - c.a);
+    uint64_t at = c.a;
+    for (uint64_t r = c.first; at < c.b && r < n_records; ++r) {
+        auto fail = [&](int code) { c.bad = r; c.code = code; };
+        const FqLine t = fq_line(text, n, at);
+        if (t.end == t.begin) { fail(cls::kFastqBlankLine); return; }
+        if (text[t.begin] != '@') { fail(cls::kFastqNoAt); return; }
+        if (t.next >= n) { fail(cls::kFastqTruncated); return; }
+        const FqLine s = fq_line(text, n, t.next);
+        if (s.next >= n) { fail(cls::kFastqTruncated); return; }
+        const FqLine p = fq_line(text, n, s.next);
+        if (p.next >= n) { fail(cls::kFastqTruncated); return; }
+        const FqLine q = fq_line(text, n, p.next);
+        if (p.end == p.begin || text[p.begin] != '+') { fail(cls::kFastqNoPlus); return; }
+        if (q.end - q.begin != s.end - s.begin) { fail(cls::kFastqQualityLength); return; }
+        bool ascii = true;
+        for (uint64_t i = t.begin + 1; i < t.end && ascii; ++i) ascii = text[i] < 0x80;
+        if (!ascii && !valid_utf8(text + t.begin + 1, t.end - t.begin - 1)) { fail(cls::kFastqTitleUtf8); return; }
+        c.hb.push_back(t.begin + 1);
+        c.he.push_back(t.end);
+        uint64_t k = 0;
+        uint8_t *out = c.bases.data() + c.kept;
+        for (uint64_t i = s.begin; i < s.end; ++i) {   // a byte rule: bytes >= 0x80 are deleted like every non-A/C/G/T byte
+            const uint8_t u = text[i] & 0xDFu;
+            if (text[i] >= 'A' && text[i] < 0x80 && (u == 'A' || u == 'C' || u == 'G' || u == 'T')) out[k++] = u;
+        }
+        c.len.push_back(k);
+        c.kept += k;
+        at = q.next;
+    }
+}
+
+}  // namespace
+
+extern "C" int cls_fastq_read(const uint8_t *text, uint64_t n_bytes, cls_fasta_text **out, cls_fasta_host_records *rec) {
+    using cls::set_last_error;
+    if (!out || !rec || (n_bytes && !text)) return set_last_error(CLS_ERR_INVALID_ARGUMENT, "NULL argument");
+    *out = nullptr;
+    memset(rec, 0, sizeof *rec);
+    try {
+        auto ft = std::make_unique<cls_fasta_text>();
+        ft->offsets.push_back(0);
+        ft->bases.reset(new uint8_t[n_bytes ? n_bytes : 1]);
+        // chunk size: 2 MiB of text (CLS_FASTA_CHUNK bytes: tests put every rule on a chunk boundary)
+        uint64_t chunk_bytes = 2u << 20;
+        if (const char *e = getenv("CLS_FASTA_CHUNK")) { const long long v = atoll(e); if (v > 0) chunk_bytes = (uint64_t)v; }
+        std::vector<FqChunk> raw;                                    // cut at line ends
+        for (uint64_t at = 0; at < n_bytes;) {
+            uint64_t end = n_bytes;
+            if (n_bytes - at > chunk_bytes) {
+                const uint8_t *nl = static_cast<const uint8_t *>(memchr(text + at + chunk_bytes - 1, '\n', n_bytes - (at + chunk_bytes - 1)));
+                if (nl) end = (uint64_t)(nl - text) + 1;
+            }
+            raw.emplace_back();
+            raw.back().a = at; raw.back().b = end;
+            at = end;
+        }
+        cls::parallel_for(raw.size(), 1, [&](uint64_t c0, uint64_t c1) {
+            for (uint64_t c = c0; c < c1; ++c) raw[c].lines = (uint64_t)std::count(text + raw[c].a, text + raw[c].b, '\n');
+        });
+        uint64_t n_newlines = 0;
+        for (FqChunk &c : raw) {                                     // move every chunk start to its first record start
+            const uint64_t skip = (4 - (n_newlines & 3)) & 3;
+            c.first = (n_newlines + 3) / 4;
+            uint64_t a = c.a;
+            for (uint64_t j = 0; j < skip && a < n_bytes; ++j) a = fq_line(text, n_bytes, a).next;
+            c.a = a;
+            n_newlines += c.lines;
+        }
+        for (size_t c = 0; c < raw.size(); ++c) {
+            raw[c].b = c + 1 < raw.size() ? raw[c + 1].a : n_bytes;
+            if (raw[c].b < raw[c].a) raw[c].b = raw[c].a;            // a chunk of fewer than four lines holds no record start
+        }
+        const uint64_t n_records = cls::fastq_n_records(text, n_bytes, n_newlines);
+        const size_t wave = (size_t)std::max(1, cls::host_threads()) * 2;
+        std::vector<FqChunk> chunks(wave);
+        uint64_t kept = 0;
+        for (size_t w0 = 0; w0 < raw.size(); w0 += wave) {
+            const size_t nc = std::min(wave, raw.size() - w0);
+            for (size_t c = 0; c < nc; ++c) { chunks[c].a = raw[w0 + c].a; chunks[c].b = raw[w0 + c].b; chunks[c].first = raw[w0 + c].first; }
+            cls::parallel_for(nc, 1, [&](uint64_t c0, uint64_t c1) {
+                for (uint64_t c = c0; c < c1; ++c) fastq_read_chunk(text, n_bytes, n_records, chunks[c]);
+            });
+            std::vector<uint64_t> dst(nc);
+            for (size_t c = 0; c < nc; ++c) {
+                const FqChunk &ch = chunks[c];
+                if (ch.bad != ~0ull) return cls::fastq_fail(ch.bad, ch.code);   // the first bad record of the file: chunks go in order
+                dst[c] = kept;
+                ft->header_begin.insert(ft->header_begin.end(), ch.hb.begin(), ch.hb.end());
+                ft->header_end.insert(ft->header_end.end(), ch.he.begin(), ch.he.end());
+                for (uint64_t l : ch.len) ft->offsets.push_back(kept += l);
+            }
+            cls::parallel_for(nc, 1, [&](uint64_t c0, uint64_t c1) {
+                for (uint64_t c = c0; c < c1; ++c)
+                    if (chunks[c].kept) memcpy(ft->bases.get() + dst[c], chunks[c].bases.data(), chunks[c].kept);
+            });
+        }
+        rec->n_records = ft->header_begin.size();
+        rec->header_begin = ft->header_begin.data();
+        rec->header_end = ft->header_end.data();
+        rec->offsets = ft->offsets.data();
+        rec->bases = ft->bases.get();
+        *out = ft.release();
+        return CLS_OK;
+    } catch (const std::bad_alloc &) {
+        return set_last_error(CLS_ERR_OUT_OF_MEMORY, "host allocation failed while reading the FASTQ text");
+    }
+}
+
 
 // ---- place_sequences as the reference spells it (core/src/use_cases/place_sequences/mod.rs:43-270): a query FASTA, an
 //      output path, the knobs -> result / error files.  cls_sequences_open does the path handling of :73-106 and reads the
@@ -920,7 +1120,9 @@ extern "C" int cls_sequences_open(const char *query_path, const char *out_file, 
     using cls::set_last_error;
     if (!out_file || !out || !batch) return set_last_error(CLS_ERR_INVALID_ARGUMENT, "NULL argument");
     *out = nullptr;
-    if (format > 1) return set_last_error(CLS_ERR_INVALID_ARGUMENT, "format must be 0 (yaml) or 1 (jsonl)");
+    const bool fastq = (format & CLS_QUERY_FASTQ) != 0;
+    format &= ~CLS_QUERY_FASTQ;
+    if (format > 1) return set_last_error(CLS_ERR_INVALID_ARGUMENT, "format must be 0 (yaml) or 1 (jsonl), optionally ORed with CLS_QUERY_FASTQ");
     try {
         auto s = std::make_unique<cls_sequences>();
         s->format = format;
@@ -950,15 +1152,17 @@ extern "C" int cls_sequences_open(const char *query_path, const char *out_file, 
         // returns Ok with nothing placed
         struct Close { FILE *f; bool own; ~Close() { if (f && own) fclose(f); } } closer{f, !use_stdin};   // also when an allocation throws
         if (!f || !read_whole(f, s->text)) s->text.clear();
-        const int rc = cls_fasta_read(reinterpret_cast<const uint8_t *>(s->text.p), s->text.n, &s->records, &s->rec);
+        const uint8_t *text = reinterpret_cast<const uint8_t *>(s->text.p);
+        const int rc = fastq ? cls_fastq_read(text, s->text.n, &s->records, &s->rec) : cls_fasta_read(text, s->text.n, &s->records, &s->rec);
         if (rc != CLS_OK) return rc;
         s->header_off.assign(s->rec.n_records + 1, 0);
         uint64_t hbytes = 0;
         for (uint64_t i = 0; i < s->rec.n_records; ++i) hbytes += s->rec.header_end[i] - s->rec.header_begin[i];
         s->headers.reserve(hbytes);
-        for (uint64_t i = 0; i < s->rec.n_records; ++i) {          // the header line minus every '>' (:102)
+        for (uint64_t i = 0; i < s->rec.n_records; ++i) {          // the header line minus every '>' (:102); a FASTQ title as it is
             const char *a = s->text.p + s->rec.header_begin[i], *e = s->text.p + s->rec.header_end[i];
-            while (a < e) {
+            if (fastq) s->headers.append(a, e);
+            while (a < e && !fastq) {
                 const char *g = static_cast<const char *>(memchr(a, '>', (size_t)(e - a)));
                 if (!g) g = e;
                 s->headers.append(a, g);

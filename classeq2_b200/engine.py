@@ -150,6 +150,15 @@ class Index:
         """``cls_fasta_upload``: parse, filter and pack a FASTA text ON THE DEVICE.  Returns ``(batch, headers,
         lengths)``: a :class:`ResidentBatch` holding the records the reference's reader would send, their
         headers (every '>' removed) and filtered lengths."""
+        return self._upload_text(text, _lib.lib.cls_fasta_upload, lambda h: h.replace(b">", b"").decode("utf-8", "replace"))
+
+    def upload_fastq(self, text: Union[bytes, bytearray, memoryview, np.ndarray]):
+        """``cls_fastq_upload``: parse, check, filter and pack a FASTQ text ON THE DEVICE (rules: ``include/classeq_b200.h``).
+        Returns ``(batch, headers, lengths)`` as :meth:`upload_fasta`, the headers as they stand after the '@'.  A malformed
+        text raises :class:`ClsError` (``CLS_ERR_INVALID_ARGUMENT``) naming its first bad record."""
+        return self._upload_text(text, _lib.lib.cls_fastq_upload, lambda h: h.decode("utf-8"))
+
+    def _upload_text(self, text, upload, header):
         arr = np.frombuffer(text, dtype=np.uint8) if not isinstance(text, np.ndarray) else np.ascontiguousarray(text, dtype=np.uint8)
         if arr.size == 0:
             arr = np.zeros(1, np.uint8)
@@ -158,13 +167,13 @@ class Index:
             n_bytes = arr.size
         h = C.c_void_p()
         rec = _lib.FastaRecords()
-        _lib.check(_lib.lib.cls_fasta_upload(self._h, arr.ctypes.data_as(_lib.u8p), n_bytes, C.byref(h), C.byref(rec)))
+        _lib.check(upload(self._h, arr.ctypes.data_as(_lib.u8p), n_bytes, C.byref(h), C.byref(rec)))
         n = int(rec.n_records)
         hb = np.ctypeslib.as_array(rec.header_begin, shape=(n,)).copy() if n else np.zeros(0, np.uint64)
         he = np.ctypeslib.as_array(rec.header_end, shape=(n,)).copy() if n else np.zeros(0, np.uint64)
         ln = np.ctypeslib.as_array(rec.length, shape=(n,)).copy() if n else np.zeros(0, np.uint32)
         raw = arr.tobytes() if n else b""
-        headers = [raw[int(a):int(b)].replace(b">", b"").decode("utf-8", "replace") for a, b in zip(hb, he)]
+        headers = [header(raw[int(a):int(b)]) for a, b in zip(hb, he)]
         return ResidentBatch._from_handle(self, h, n), headers, ln
 
     def debug_node_counts(self, seq, params: Optional[PlaceParams] = None, cap: int = 1 << 16):

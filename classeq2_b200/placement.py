@@ -112,6 +112,88 @@ def read_fasta(query: Union[str, os.PathLike, io.TextIOBase]) -> List[Tuple[str,
 
 
 # --------------------------------------------------------------------------------------------------
+# FASTQ reading (the rules are stated in include/classeq_b200.h, above cls_fastq_upload)
+# --------------------------------------------------------------------------------------------------
+FASTQ_REASONS = {
+    1: "blank line inside the records",
+    2: "title line does not start with '@'",
+    3: "truncated record (fewer than four lines)",
+    4: "separator line does not start with '+'",
+    5: "quality length differs from sequence length",
+    6: "title is not valid UTF-8",
+}
+_FASTQ_KEEP = bytes(range(256)).translate(bytes.maketrans(b"acgt", b"ACGT"))   # ASCII upper-casing of a/c/g/t
+_FASTQ_DROP = bytes(c for c in range(256) if c not in b"ACGTacgt")
+
+
+def read_fastq_text(data: Union[bytes, bytearray, memoryview, str]) -> List[Tuple[str, str]]:
+    """The (header, sequence) records of a FASTQ text, in order: four lines per record, the header is the title line
+    after its '@', the sequence line keeps its A/C/G/T bytes (either case) and loses every other byte.  A malformed text
+    raises :class:`ClsError` (``CLS_ERR_INVALID_ARGUMENT``) with the message ``cls_fastq_read`` gives for it."""
+    raw = data.encode("utf-8") if isinstance(data, str) else bytes(data)
+    lines = raw.split(b"\n")
+    terminated = [True] * len(lines)
+    terminated[-1] = False          # what follows the last "\n" (possibly nothing) has no terminator
+    if lines[-1] == b"":
+        lines.pop()
+        terminated.pop()
+    lines = [ln[:-1] if term and ln.endswith(b"\r") else ln for ln, term in zip(lines, terminated)]
+    last = max((i for i, ln in enumerate(lines) if ln), default=-1)     # blank lines may only follow the last record
+    out: List[Tuple[str, str]] = []
+    for r in range(last // 4 + 1 if last >= 0 else 0):
+        def bad(code: int):
+            return _lib.ClsError(_lib.CLS_ERR_INVALID_ARGUMENT, f"malformed FASTQ record {r + 1}: {FASTQ_REASONS[code]}")
+        title = lines[4 * r]
+        if not title:
+            raise bad(1)
+        if not title.startswith(b"@"):
+            raise bad(2)
+        if 4 * r + 3 >= len(lines):
+            raise bad(3)
+        seq, sep, qual = lines[4 * r + 1: 4 * r + 4]
+        if not sep.startswith(b"+"):
+            raise bad(4)
+        if len(qual) != len(seq):
+            raise bad(5)
+        try:
+            header = title[1:].decode("utf-8")
+        except UnicodeDecodeError:
+            raise bad(6) from None
+        out.append((header, seq.translate(_FASTQ_KEEP, _FASTQ_DROP).decode("ascii")))
+    return out
+
+
+def read_fastq_native(data: Union[bytes, bytearray, memoryview, str]) -> Tuple[List[str], np.ndarray, np.ndarray]:
+    """``cls_fastq_read``: the FASTQ reader in the library.  Returns ``(headers, bases, offsets)`` as
+    :func:`read_fasta_native` - the records :func:`read_fastq_text` returns."""
+    raw = data.encode("utf-8") if isinstance(data, str) else bytes(data)
+    arr = np.frombuffer(raw, dtype=np.uint8) if raw else np.zeros(1, np.uint8)
+    h, rec = C.c_void_p(), _lib.FastaHostRecords()
+    _lib.check(_lib.lib.cls_fastq_read(arr.ctypes.data_as(_lib.u8p), len(raw), C.byref(h), C.byref(rec)))
+    try:
+        n = int(rec.n_records)
+        offsets = np.ctypeslib.as_array(rec.offsets, shape=(n + 1,)).copy()
+        total = int(offsets[-1])
+        bases = np.ctypeslib.as_array(rec.bases, shape=(max(total, 1),))[:total].copy()
+        hb = np.ctypeslib.as_array(rec.header_begin, shape=(n,)).tolist() if n else []
+        he = np.ctypeslib.as_array(rec.header_end, shape=(n,)).tolist() if n else []
+    finally:
+        _lib.lib.cls_fasta_text_destroy(h)
+    headers = [raw[a:b].decode("utf-8") for a, b in zip(hb, he)]
+    return headers, bases, offsets
+
+
+def read_fastq(query: Union[str, os.PathLike, io.IOBase]) -> List[Tuple[str, str]]:
+    """:func:`read_fastq_text` on a path, ``"-"`` for stdin, or an open stream."""
+    if hasattr(query, "read"):
+        return read_fastq_text(query.read())
+    if str(query) == "-":
+        return read_fastq_text(sys.stdin.buffer.read())
+    with open(query, "rb") as f:
+        return read_fastq_text(f.read())
+
+
+# --------------------------------------------------------------------------------------------------
 # serde-compatible emitters (serde_yaml 0.9 / serde_json 1.0 with ryu float formatting)
 # --------------------------------------------------------------------------------------------------
 def ryu_float(x: float) -> str:
@@ -657,7 +739,7 @@ def place_sequences(query_sequence, tree: Tree, out_file: Union[str, os.PathLike
                     overwrite: bool = False, output_format: str = "yaml",
                     remove_intersection: Optional[bool] = None, *, index: Optional[Index] = None,
                     device: int = 0, batch_size: int = 1 << 20, ingest: str = "host",
-                    writer: str = "native", reader: str = "native") -> List[PlacementTime]:
+                    writer: str = "native", reader: str = "native", query_format: str = "fasta") -> List[PlacementTime]:
     """Place every sequence of a FASTA input on ``tree`` and append one record per query to
     ``<out_file>.yaml|.jsonl`` (errors to ``<out_file>.error``), as the reference does.
 
@@ -669,9 +751,15 @@ def place_sequences(query_sequence, tree: Tree, out_file: Union[str, os.PathLike
     ``writer="python"`` uses this module's emitters - the two write byte-identical files (tests/test_record_writer.py).
     ``reader="native"`` (default, host ingest) parses the FASTA text in the library (``cls_fasta_read``); ``"python"``
     uses :func:`read_fasta_text` - the same records (tests/test_fasta_reader.py).
+    ``query_format="fastq"`` reads the query as FASTQ (rules: ``include/classeq_b200.h``) with every ingest and reader:
+    ``cls_fastq_upload``, ``cls_fastq_read`` or :func:`read_fastq_text`.  A malformed FASTQ raises :class:`ClsError`
+    before either file is created.
     """
     if writer not in ("native", "python") or reader not in ("native", "python"):
         raise ValueError("writer / reader must be 'native' or 'python'")
+    if query_format not in ("fasta", "fastq"):
+        raise ValueError("query_format must be 'fasta' or 'fastq'")
+    fastq = query_format == "fastq"
     if ingest not in ("host", "device"):
         raise ValueError("ingest must be 'host' or 'device'")
     if output_format not in ("yaml", "jsonl"):
@@ -703,7 +791,12 @@ def place_sequences(query_sequence, tree: Tree, out_file: Union[str, os.PathLike
                 raw = f.read()
         except OSError:
             raw = b""                                                          # nothing placed, no error (see below)
-        device_batch, headers, _ = index.upload_fasta(raw)
+        try:
+            device_batch, headers, _ = index.upload_fastq(raw) if fastq else index.upload_fasta(raw)
+        except BaseException:
+            if own_index:
+                index.close()
+            raise
         records = [(h, None) for h in headers]
         batch_size = max(len(records), 1)
     elif reader == "native":
@@ -720,13 +813,22 @@ def place_sequences(query_sequence, tree: Tree, out_file: Union[str, os.PathLike
                 # Result (`let _ = query_sequence.sequence_content_by_channel(sender)`, mod.rs:119), has created both files
                 # by then (:111-115) and returns Ok with nothing placed - as cls_sequences_open does
                 raw = b""
-        headers, host_bases, host_offsets = read_fasta_native(raw)
+        try:
+            headers, host_bases, host_offsets = read_fastq_native(raw) if fastq else read_fasta_native(raw)
+        except BaseException:
+            if own_index:
+                index.close()
+            raise
         records = [(h, None) for h in headers]
     else:
         try:
-            records = read_fasta(query_sequence)
+            records = read_fastq(query_sequence) if fastq else read_fasta(query_sequence)
         except OSError:
             records = []
+        except BaseException:
+            if own_index:
+                index.close()
+            raise
     lookup = _TreeLookup(tree) if writer == "python" else None
     rtree = RecordTree(tree) if writer == "native" else None
     params = PlaceParams(max_iterations, min_match_coverage, remove_intersection)
@@ -774,12 +876,16 @@ def place_sequences(query_sequence, tree: Tree, out_file: Union[str, os.PathLike
 def place_sequences_native(query_sequence: Union[str, os.PathLike], tree: Tree, out_file: Union[str, os.PathLike],
                            max_iterations: Optional[int] = None, min_match_coverage: Optional[float] = None,
                            overwrite: bool = False, output_format: str = "yaml",
-                           remove_intersection: Optional[bool] = None, *, index: Optional[Index] = None, device: int = 0) -> int:
-    """The whole use-case in ONE library call (``cls_place_sequences``): path handling, FASTA reader, placement on the GPU
-    and record writer all run in the library; this wrapper only flattens the tree.  Same arguments as
+                           remove_intersection: Optional[bool] = None, *, index: Optional[Index] = None, device: int = 0,
+                           query_format: str = "fasta") -> int:
+    """The whole use-case in ONE library call (``cls_place_sequences``): path handling, FASTA or FASTQ reader, placement on
+    the GPU and record writer all run in the library; this wrapper only flattens the tree.  Same arguments as
     :func:`place_sequences` (a path or ``"-"`` for stdin), same files.  Returns the number of records placed."""
     if output_format not in ("yaml", "jsonl"):
         raise ValueError("output_format must be 'yaml' or 'jsonl'")
+    if query_format not in ("fasta", "fastq"):
+        raise ValueError("query_format must be 'fasta' or 'fastq'")
+    fmt = (0 if output_format == "yaml" else 1) | (_lib.QUERY_FASTQ if query_format == "fastq" else 0)
     own_index = index is None
     if own_index:
         index = Index(tree, device=device)
@@ -788,7 +894,7 @@ def place_sequences_native(query_sequence: Union[str, os.PathLike], tree: Tree, 
         params = PlaceParams(max_iterations, min_match_coverage, remove_intersection).to_c()
         n = C.c_uint64()
         rc = _lib.lib.cls_place_sequences(index._h, C.byref(rtree.view), os.fspath(query_sequence).encode(), os.fspath(out_file).encode(),
-                                          C.byref(params), 0 if output_format == "yaml" else 1, 1 if overwrite else 0, C.byref(n))
+                                          C.byref(params), fmt, 1 if overwrite else 0, C.byref(n))
         if rc == _lib.CLS_ERR_INVALID_ARGUMENT and _lib.last_error().startswith("Could not overwrite existing file"):
             raise FileExistsError(_lib.last_error())
         _lib.check(rc)

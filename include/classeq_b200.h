@@ -282,6 +282,31 @@ int cls_fasta_upload(cls_index *index, const uint8_t *text, uint64_t n_bytes, cl
                      cls_fasta_records *records);
 
 /*
+ * FASTQ queries.  The reference reads only FASTA; these rules make a FASTQ file and its FASTA rendering (">" + title,
+ * then the sequence line) place identically, for titles that are not empty and hold no '>', and a last record with at
+ * least one base.  Lines end at "\n"; a "\r" right before the "\n" belongs to the terminator; the last line may lack one.
+ * A record is exactly four lines (wrapped multi-line FASTQ is malformed):
+ *   1. the title line starts with '@'; the header is the rest of the line, byte for byte (one '@' removed, nothing else);
+ *   2. the sequence line, filtered as a FASTA sequence line: ASCII letters upper-cased, A/C/G/T kept, every other byte
+ *      (N, IUPAC codes, '.', '-', bytes >= 0x80) deleted and the flanks joined;
+ *   3. the separator line starts with '+'; the rest of it is ignored;
+ *   4. the quality line has as many bytes as the sequence line (terminator excluded); its content is not used.
+ * Every well-formed record is sent, also one whose filtered sequence is empty or shorter than k (it becomes
+ * CLS_STATUS_ERR_TOO_SHORT) and one whose title is '@' alone (empty header).  Blank lines may follow the last record only.
+ * A malformed file is refused as a whole with CLS_ERR_INVALID_ARGUMENT, nothing placed or written, and cls_last_error()
+ * names the first bad record ("malformed FASTQ record <1-based number>: <reason>"): a title line without '@', a separator
+ * line without '+', a quality length that differs from the sequence length, a blank line among the records, a truncated
+ * last record, a title that is not valid UTF-8 (headers are written as UTF-8 text).
+ *
+ * cls_fastq_upload: FASTQ ingest on the device, as cls_fasta_upload: the resident batch cls_batch_upload would have built
+ * from cls_fastq_read's records, in record order; header = text[header_begin .. header_end) as it is (header_begin is one
+ * past the '@').  Works on the first device of a multi-device or sharded handle.  Texts of 4 GiB or more are
+ * CLS_ERR_UNSUPPORTED.
+ */
+int cls_fastq_upload(cls_index *index, const uint8_t *text, uint64_t n_bytes, cls_resident_batch **out,
+                     cls_fasta_records *records);
+
+/*
  * Hash-sharded index (config 5 of BASELINE.json; SURVEY.md section 8e).  The k-mer table is split over up
  * to 8 GPUs by `owner = (hash >> 61) % n_shards`; node-set records and the tree are replicated.
  * The reference has no counterpart (its index is one in-memory HashMap, kmers_map.rs:77-87): these
@@ -468,6 +493,9 @@ typedef struct cls_fasta_host_records {
 } cls_fasta_host_records;
 int cls_fasta_read(const uint8_t *text, uint64_t n_bytes, cls_fasta_text **out, cls_fasta_host_records *records);
 void cls_fasta_text_destroy(cls_fasta_text *t);
+/* The FASTQ reader on the host (rules above cls_fastq_upload): header = text[header_begin .. header_end) as it is.  The
+ * handle is released with cls_fasta_text_destroy. */
+int cls_fastq_read(const uint8_t *text, uint64_t n_bytes, cls_fasta_text **out, cls_fasta_host_records *records);
 
 /*
  * `place_sequences` as the reference spells it (core/src/use_cases/place_sequences/mod.rs:43-53): a query FASTA (path,
@@ -478,7 +506,11 @@ void cls_fasta_text_destroy(cls_fasta_text *t);
  *                          reference's message) + the reader (:118-119); `batch` receives a borrowed view of the records
  *   cls_sequences_write    appends the records / error texts of the next `n` results (in record order) to the two files
  * The split exists for callers that place on their own schedule (several GPUs, resident batches) and for tests.
+ * `format` is 0 (yaml) or 1 (jsonl), ORed with CLS_QUERY_FASTQ to read the query as FASTQ (cls_fastq_read; its headers
+ * are written as they are, while FASTA headers lose every '>').  A malformed FASTQ query is CLS_ERR_INVALID_ARGUMENT
+ * before either file is created.
  */
+#define CLS_QUERY_FASTQ 0x100u
 typedef struct cls_sequences cls_sequences;
 int cls_sequences_open(const char *query_path, const char *out_file, uint32_t format, uint32_t overwrite,
                        cls_sequences **out, cls_batch *batch);
