@@ -24,11 +24,8 @@
 #include "build_prep.hpp"
 #include "build_steps.hpp"
 #include "built_model.hpp"
+#include "last_error.hpp"
 #include "murmur3_device.cuh"
-
-namespace cls {
-int set_last_error(int code, const std::string &msg);  // capi.cu
-}
 
 namespace {
 

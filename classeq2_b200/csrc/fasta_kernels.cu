@@ -7,7 +7,7 @@
 //     everything else - N, IUPAC codes, gaps, blanks - is DELETED and the flanks are joined.
 // The device does the per-byte work (classification, filtering, compaction, packing) with two
 // reduce-then-scan passes over 4 KiB tiles; the record-level rules (empty headers, the trailing
-// record, "sequence without header") are a few comparisons per record on the host (capi.cu).
+// record, "sequence without header") are a few comparisons per record on the host (resident.cpp).
 // Non-ASCII bytes are reported, not interpreted: Rust's to_uppercase() maps a handful of non-ASCII
 // scalars to strings containing A/C/G/T, and the caller then uses the host reader.
 #include <cuda_runtime.h>

@@ -1,4 +1,4 @@
-// Launch interface of the FASTA ingest kernels (fasta_kernels.cu), used by cls_fasta_upload (capi.cu).
+// Launch interface of the FASTA ingest kernels (fasta_kernels.cu), used by cls_fasta_upload (resident.cpp).
 #pragma once
 #include <cuda_runtime.h>
 

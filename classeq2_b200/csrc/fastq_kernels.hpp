@@ -1,4 +1,4 @@
-// Launch interface of the FASTQ ingest kernels (fastq_kernels.cu), used by cls_fastq_upload (capi.cu).
+// Launch interface of the FASTQ ingest kernels (fastq_kernels.cu), used by cls_fastq_upload (fastq_ingest.cpp).
 #pragma once
 #include <cuda_runtime.h>
 

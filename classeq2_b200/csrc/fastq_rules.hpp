@@ -1,5 +1,5 @@
 // What the two FASTQ readers share: the host reader cls_fastq_read (record_writer.cpp) and the device ingest
-// cls_fastq_upload (capi.cu, fastq_kernels.cu) refuse a malformed file with the same first bad record and reason.
+// cls_fastq_upload (fastq_ingest.cpp, fastq_kernels.cu) refuse a malformed file with the same first bad record and reason.
 #pragma once
 #include <cstdint>
 

@@ -17,6 +17,7 @@
 #include "../../include/classeq_b200.h"
 #include "built_model.hpp"
 #include "host_pool.hpp"
+#include "last_error.hpp"
 #include "murmur3_host.hpp"
 
 namespace {
@@ -30,16 +31,6 @@ struct Occ {
 inline uint64_t mix64(uint64_t x) { return cls::fmix64_h(x + 0x9e3779b97f4a7c15ULL); }
 
 }  // namespace
-
-extern "C" {
-
-// defined in capi.cu
-const char *cls_last_error(void);
-}
-
-namespace cls {
-int set_last_error(int code, const std::string &msg);  // capi.cu
-}
 
 static int build_host(const cls_model_view *tree, uint64_t n_tips, const uint64_t *tip_node,
                       const uint8_t *bases, const uint64_t *offsets, cls_built_model **out) {

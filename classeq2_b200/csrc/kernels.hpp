@@ -1,4 +1,4 @@
-// Launch interface of the sm_100a kernels (kernels.cu), used by the C-ABI layer (capi.cu).
+// Launch interface of the sm_100a kernels (kernels.cu), used by the C-ABI layer (capi_internal.hpp).
 #pragma once
 #include <cuda_runtime.h>
 

@@ -35,10 +35,7 @@
 #include "../../include/classeq_b200.h"
 #include "fastq_rules.hpp"
 #include "host_pool.hpp"
-
-namespace cls {
-int set_last_error(int code, const std::string &msg);  // capi.cu
-}
+#include "last_error.hpp"
 
 namespace {
 

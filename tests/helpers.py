@@ -1,5 +1,13 @@
-"""Comparison helpers shared by the parity tests."""
+"""Comparison helpers shared by the parity tests, and the host sources the fake-runtime drivers compile."""
+import os
+
 from classeq2_b200 import _lib
+
+CSRC = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "classeq2_b200", "csrc")
+# The C ABI's host side without the sharded handle (capi_sharded.cpp) and the FASTQ ingest (fastq_ingest.cpp), which the
+# drivers that need them add: compiled with g++ against the fake CUDA runtime of tests/native/fakecuda.
+CAPI_HOST_SOURCES = [os.path.join(CSRC, f) for f in ("capi.cpp", "place_batch.cpp", "resident.cpp", "routed.cpp", "index_build.cpp",
+                                                     "host_api.cpp", "host_pack.cpp", "host_pool.cpp", "record_writer.cpp")]
 
 UNCL_BY_MESSAGE_PREFIX = {
     "Query sequence SequenceHeader(": _lib.STATUS_UNCL_NO_MATCH,

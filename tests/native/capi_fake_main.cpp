@@ -1,4 +1,4 @@
-// TEST INFRASTRUCTURE.  cls_place_batch and its neighbours (classeq2_b200/csrc/capi.cu) end to end WITHOUT a GPU: the
+// TEST INFRASTRUCTURE.  cls_place_batch and its neighbours (classeq2_b200/csrc/place_batch.cpp) end to end WITHOUT a GPU: the
 // library's host side is compiled against the fake CUDA runtime (tests/native/fakecuda/) and the placement launch hands
 // the reads it was given - unpacked from the 2-bit words at their descriptors - to the C++ oracle
 // (tests/native/fake_kernels.cpp).  The results must equal the oracle's on the caller's ASCII batch, for every way the

@@ -1,5 +1,5 @@
 // TEST INFRASTRUCTURE.  The launch functions of kernels.hpp / fasta_kernels.hpp for the fake CUDA runtime
-// (tests/native/fakecuda/cuda_runtime.h), so that capi.cu runs without a GPU:
+// (tests/native/fakecuda/cuda_runtime.h), so that the C ABI's host side runs without a GPU:
 //   launch_place        unpacks every read of the launch from the 2-bit words at its descriptor and hands it to the C++
 //                       oracle (oracle/classeq_oracle.cpp, linked into the test) - what the placement kernels compute,
 //                       by other means; the result records land where the kernels would write them;

@@ -1,7 +1,7 @@
 // TEST INFRASTRUCTURE.  The peer-access calls of the CUDA runtime on top of the fake runtime (tests/native/fakecuda/):
 // every pair of distinct fake devices can reach each other (FAKE_CUDA_NO_PEER=1: none can); enabling a pair twice
 // reports cudaErrorPeerAccessAlreadyEnabled, as the real runtime does.  Force-included (-include) into
-// classeq2_b200/csrc/capi_sharded.cu by tests/test_sharded_handle.py.
+// classeq2_b200/csrc/capi_sharded.cpp by tests/test_sharded_handle.py.
 #pragma once
 #include <cuda_runtime.h>
 

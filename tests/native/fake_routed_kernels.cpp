@@ -1,5 +1,5 @@
 // TEST INFRASTRUCTURE.  The launch functions of tests/native/fake_kernels.cpp with its routed stubs replaced by host
-// restatements of the routed kernels (routed_kernels.cuh), for the sharded handle (classeq2_b200/csrc/capi_sharded.cu)
+// restatements of the routed kernels (routed_kernels.cuh), for the sharded handle (classeq2_b200/csrc/capi_sharded.cpp)
 // without a GPU:
 //   launch_route                hashes every window with the oracle's hash and appends it to its owner's segment (one run
 //                               per read and owner, the window behind every slot, the cursors, the overflow flag) as

@@ -1,5 +1,5 @@
 // TEST INFRASTRUCTURE.  A stand-in for <cuda_runtime.h> that lets the HOST side of the library (classeq2_b200/csrc/
-// capi.cu: planning, packing, chunked pipeline, scatter, multi-device fan-out, workspaces) compile with g++ and run
+// capi.cpp and its neighbours: planning, packing, chunked pipeline, scatter, multi-device fan-out) compile with g++ and run
 // without a GPU, under AddressSanitizer / ThreadSanitizer.  "Device" memory is malloc'ed host memory (so a copy that
 // runs past a device buffer is an ASan report), events carry the host clock.  Two modes:
 //   * synchronous (default): every "asynchronous" call completes before it returns - the host logic, its buffer sizes

@@ -1,4 +1,4 @@
-// TEST INFRASTRUCTURE.  The host side of cls_fastq_upload (classeq2_b200/csrc/fastq_ingest.cpp, capi.cu) WITHOUT a GPU: compiled against the
+// TEST INFRASTRUCTURE.  The host side of cls_fastq_upload (classeq2_b200/csrc/fastq_ingest.cpp, resident.cpp) WITHOUT a GPU: compiled against the
 // fake CUDA runtime (tests/native/fakecuda/), with fastq_kernels.cu's launches restated as serial walks
 // (fake_fastq_kernels.cpp) and the placement launch answered by the C++ oracle (fake_kernels.cpp).  On random and
 // hand-made FASTQ texts the upload must give cls_fastq_read's records (header slices, lengths) and the placements

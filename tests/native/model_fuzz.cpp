@@ -13,7 +13,7 @@
 #include "../../classeq2_b200/csrc/murmur3_host.hpp"
 
 namespace cls {
-int set_last_error(int code, const std::string &) { return code; }   // capi.cu's, stubbed
+int set_last_error(int code, const std::string &) { return code; }   // capi.cpp's, stubbed
 }
 extern "C" uint64_t cls_debug_host_murmur3_x64_128_h1(const uint8_t *d, uint64_t n, uint64_t s) { return cls::murmur3_x64_128_h1(d, n, s); }
 extern "C" const char *cls_last_error(void) { return ""; }

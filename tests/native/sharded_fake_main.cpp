@@ -1,4 +1,4 @@
-// TEST INFRASTRUCTURE.  The sharded handle (cls_index_create_sharded, classeq2_b200/csrc/capi_sharded.cu) end to end WITHOUT a GPU:
+// TEST INFRASTRUCTURE.  The sharded handle (cls_index_create_sharded, classeq2_b200/csrc/capi_sharded.cpp) end to end WITHOUT a GPU:
 // the library's host side against the fake CUDA runtime (tests/native/fakecuda/), the three routed launches restated on the
 // host (tests/native/fake_routed_kernels.cpp: route with the oracle's hash, probe over the shard's uploaded table, place_routed
 // checking every reply against a direct probe of the owner shard before the oracle places the read).  Results must equal

@@ -13,10 +13,10 @@
 #include "../../include/classeq_b200.h"
 
 namespace cls {
-int set_last_error(int code, const std::string &) { return code; }   // capi.cu's, stubbed
+int set_last_error(int code, const std::string &) { return code; }   // capi.cpp's, stubbed
 }
 extern "C" int cls_place_batch(cls_index *, const cls_batch *, const cls_params *, cls_result *) { return CLS_ERR_CUDA; }  // no device here
-extern "C" const char *cls_last_error(void) { return ""; }   // capi.cu's (cls_place_sequences carries the writer thread's message over)
+extern "C" const char *cls_last_error(void) { return ""; }   // capi.cpp's (cls_place_sequences carries the writer thread's message over)
 
 static uint64_t rng_state = 88172645463325252ull;
 static uint64_t rnd() { rng_state ^= rng_state << 13; rng_state ^= rng_state >> 7; rng_state ^= rng_state << 17; return rng_state; }

@@ -1,7 +1,8 @@
-"""The HOST side of the hot path's public call - ``cls_place_batch`` and its neighbours in classeq2_b200/csrc/capi.cu:
+"""The HOST side of the hot path's public call - ``cls_place_batch`` and its neighbours (classeq2_b200/csrc/capi.cpp,
+place_batch.cpp, resident.cpp, routed.cpp):
 planning (general and just in time, with its fallback), host / device / mixed packing from pageable and pinned memory,
 the chunked pipeline, scatter into the caller's arrays, resident batches, one handle over several devices, concurrent
-callers, a failing launch - end to end WITHOUT a GPU.  capi.cu is compiled with g++ against a fake CUDA runtime
+callers, a failing launch - end to end WITHOUT a GPU.  They are compiled with g++ against a fake CUDA runtime
 (tests/native/fakecuda/cuda_runtime.h: device memory is host memory, every call completes before it returns); the
 placement launch unpacks the reads it is handed and gives them to the C++ oracle (tests/native/fake_kernels.cpp); the
 results must equal the oracle's on the caller's ASCII batch (tests/native/capi_fake_main.cpp).  Run under
@@ -13,13 +14,12 @@ import subprocess
 
 import pytest
 
+from helpers import CAPI_HOST_SOURCES
+
 HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(HERE)
-CSRC = os.path.join(ROOT, "classeq2_b200", "csrc")
 FAKE = os.path.join(HERE, "native", "fakecuda")
-SOURCES = [(os.path.join(CSRC, "capi.cu"), True)] + [(os.path.join(CSRC, f), False) for f in
-                                                      ("index_build.cpp", "host_api.cpp", "host_pack.cpp", "host_pool.cpp", "record_writer.cpp")] + \
-          [(os.path.join(HERE, "native", f), False) for f in ("capi_fake_main.cpp", "fake_kernels.cpp")]
+SOURCES = CAPI_HOST_SOURCES + [os.path.join(HERE, "native", f) for f in ("capi_fake_main.cpp", "fake_kernels.cpp")]
 
 
 def _compile(tmp_path, name, san):
@@ -33,10 +33,10 @@ def _compile(tmp_path, name, san):
         _compile.orc_started = True
         jobs.append(subprocess.Popen(["g++", "-O2", "-std=c++17", "-pthread", "-c", os.path.join(ROOT, "oracle", "classeq_oracle.cpp"), "-o", str(orc)],
                                      stderr=subprocess.PIPE, text=True))
-    for src, is_cu in SOURCES:
+    for src in SOURCES:
         obj = str(out / (os.path.basename(src) + ".o"))
         objs.append(obj)
-        cmd = ["g++", "-O1", "-g", "-std=c++17", "-pthread", *san, "-I", FAKE] + (["-x", "c++"] if is_cu else []) + ["-c", src, "-o", obj]
+        cmd = ["g++", "-O1", "-g", "-std=c++17", "-pthread", *san, "-I", FAKE, "-c", src, "-o", obj]
         jobs.append(subprocess.Popen(cmd, stderr=subprocess.PIPE, text=True))
     return jobs, objs, str(orc), str(out / "capi_fake"), san
 

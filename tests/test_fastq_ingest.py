@@ -8,6 +8,8 @@ import subprocess
 import numpy as np
 import pytest
 
+from helpers import CAPI_HOST_SOURCES, CSRC
+
 HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(HERE)
 GOLDEN = os.path.join(HERE, "golden")
@@ -201,23 +203,22 @@ def test_sequences_open_with_fastq_flag(tmp_path):
 
 # ---- the host side of cls_fastq_upload against a fake CUDA runtime, under ASan + UBSan ---------------------------------
 def test_fastq_upload_host_side_under_asan(tmp_path):
-    """capi.cu and fastq_ingest.cpp compiled with g++ against tests/native/fakecuda, the FASTQ kernels restated as serial walks
+    """The C ABI's host sources and fastq_ingest.cpp compiled with g++ against tests/native/fakecuda, the FASTQ kernels restated as serial walks
     (tests/native/fake_fastq_kernels.cpp): cls_fastq_upload's host side (record count, first bad record, UTF-8 titles,
     lengths, planning, packing) gives cls_fastq_read's records and, through the oracle, the same placements."""
     if shutil.which("g++") is None:
         pytest.skip("needs g++")
-    csrc, native = os.path.join(ROOT, "classeq2_b200", "csrc"), os.path.join(HERE, "native")
+    native = os.path.join(HERE, "native")
     orc, exe = str(tmp_path / "oracle.o"), str(tmp_path / "fastq_fake")
     # the oracle is the checker: compiled once, without a sanitizer (its allocations would dominate the run under one)
     r = subprocess.run(["g++", "-O2", "-std=c++17", "-pthread", "-c", os.path.join(ROOT, "oracle", "classeq_oracle.cpp"), "-o", orc],
                        capture_output=True, text=True)
     assert r.returncode == 0, r.stderr[-3000:]
     san = ["-fsanitize=address,undefined", "-fno-sanitize-recover=undefined"]
-    srcs = [os.path.join(csrc, f) for f in ("index_build.cpp", "host_api.cpp", "host_pack.cpp", "host_pool.cpp", "record_writer.cpp",
-                                             "fastq_ingest.cpp")] + \
+    srcs = CAPI_HOST_SOURCES + [os.path.join(CSRC, "fastq_ingest.cpp")] + \
            [os.path.join(native, f) for f in ("fastq_fake_main.cpp", "fake_kernels.cpp", "fake_fastq_kernels.cpp")]
-    r = subprocess.run(["g++", "-O1", "-g", "-std=c++17", "-pthread", *san, "-I", os.path.join(native, "fakecuda"),
-                        "-x", "c++", os.path.join(csrc, "capi.cu"), "-x", "none", *srcs, orc, "-o", exe], capture_output=True, text=True)
+    r = subprocess.run(["g++", "-O1", "-g", "-std=c++17", "-pthread", *san, "-I", os.path.join(native, "fakecuda"), *srcs, orc, "-o", exe],
+                       capture_output=True, text=True)
     assert "error:" not in r.stderr and "undefined reference" not in r.stderr, r.stderr[-3000:]   # a real build error is a failure
     if r.returncode != 0:
         pytest.skip(f"cannot build with the sanitizers here: {r.stderr[-300:]}")

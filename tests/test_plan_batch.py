@@ -1,4 +1,4 @@
-"""The host-side planner of ``cls_place_batch`` / ``cls_batch_upload`` (capi.cu: plan_batch) through
+"""The host-side planner of ``cls_place_batch`` / ``cls_batch_upload`` (place_batch.cpp: plan_batch) through
 ``cls_debug_plan_batch``: host-decided statuses, length classes, device order and packed layout.  No GPU."""
 import ctypes as C
 
@@ -30,7 +30,7 @@ def plan(lens, k):
 
 
 def class_of(length, k):
-    """Table geometry shared by a class: log2 of the de-duplication table size for that length (capi.cu)."""
+    """Table geometry shared by a class: log2 of the de-duplication table size for that length (place_batch.cpp)."""
     h2, c = 4 * (length - k + 1), 6
     while (1 << c) < h2:
         c += 1
@@ -98,7 +98,7 @@ def test_plan_degenerate_batches():
     assert rc == _lib.CLS_ERR_INVALID_ARGUMENT
 
 
-# ---- the just-in-time plan of short-read batches (capi.cu: plan_reads_fast) --------------------------------------
+# ---- the just-in-time plan of short-read batches (place_batch.cpp: plan_reads_fast) ---------------------------------
 def plan_fast(lens, k, chunk, first_offset=0):
     lens = np.asarray(lens, np.uint64)
     n = len(lens)

@@ -5,7 +5,7 @@ well; the test with one shard per visible GPU skips below two.
 
 Without a GPU the host side runs against the fake CUDA runtime (tests/native/sharded_fake_main.cpp, the peer-access
 calls in tests/native/fake_peer_runtime.h, the routed launches restated in tests/native/fake_routed_kernels.cpp) under AddressSanitizer + UBSan and, with every stream a worker thread, under
-ThreadSanitizer.  Dropping the owner's wait for a sender's route event (enqueue_routed in capi_sharded.cu) makes ThreadSanitizer
+ThreadSanitizer.  Dropping the owner's wait for a sender's route event (enqueue_routed in capi_sharded.cpp) makes ThreadSanitizer
 report races there (checked by mutation)."""
 import os
 import shutil
@@ -15,14 +15,13 @@ import threading
 import numpy as np
 import pytest
 
+from helpers import CAPI_HOST_SOURCES, CSRC
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(HERE)
-CSRC = os.path.join(ROOT, "classeq2_b200", "csrc")
 FIELDS = ("status", "node_id", "one", "rest", "n_query_kmers", "n_matched", "n_root_matched", "iterations")
-SOURCES = [(os.path.join(CSRC, "capi_sharded.cu"), True)] + [(os.path.join(CSRC, f), False) for f in
-                                                              ("index_build.cpp", "host_api.cpp", "host_pack.cpp", "host_pool.cpp", "record_writer.cpp")] + \
-          [(os.path.join(HERE, "native", f), False) for f in ("sharded_fake_main.cpp", "fake_routed_kernels.cpp")]
+SHARDED = os.path.join(CSRC, "capi_sharded.cpp")
+SOURCES = [SHARDED] + CAPI_HOST_SOURCES + [os.path.join(HERE, "native", f) for f in ("sharded_fake_main.cpp", "fake_routed_kernels.cpp")]
 
 
 # ---- host side on the fake runtime ------------------------------------------------------------------------------------------
@@ -30,11 +29,11 @@ def _build(tmp, name, san, orc):
     out = tmp / name
     out.mkdir()
     jobs, objs = [], []
-    for src, is_cu in SOURCES:
+    for src in SOURCES:
         obj = str(out / (os.path.basename(src) + ".o"))
         objs.append(obj)
         cmd = ["g++", "-O1", "-g", "-std=c++17", "-pthread", *san, "-I", os.path.join(HERE, "native", "fakecuda")] + \
-              (["-x", "c++", "-include", os.path.join(HERE, "native", "fake_peer_runtime.h")] if is_cu else []) + ["-c", src, "-o", obj]
+              (["-include", os.path.join(HERE, "native", "fake_peer_runtime.h")] if src == SHARDED else []) + ["-c", src, "-o", obj]
         jobs.append(subprocess.Popen(cmd, stderr=subprocess.PIPE, text=True))
     for p in jobs:
         _, err = p.communicate()

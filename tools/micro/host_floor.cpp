@@ -1,8 +1,8 @@
-// Host-side cost of one cls_place_batch call with the GPU taken out: capi.cu against the fake CUDA runtime of the tests
+// Host-side cost of one cls_place_batch call with the GPU taken out: the C ABI's host side against the fake CUDA runtime of the tests
 // (tests/native/fakecuda/), copies and kernels costing nothing - what remains is planning, 2-bit packing or staging,
 // descriptors, and the scatter of the result records into the caller's arrays, on this machine's cores.  On a GPU box
 // this work runs next to the kernels: it is exposed only where it exceeds them (several GPUs sharing few cores).
-//   g++ -O2 -std=c++17 -pthread -Itests/native/fakecuda -x c++ classeq2_b200/csrc/capi.cu -x none tools/micro/host_floor.cpp \
+//   g++ -O2 -std=c++17 -pthread -Itests/native/fakecuda classeq2_b200/csrc/{capi,place_batch,resident,routed}.cpp tools/micro/host_floor.cpp \
 //       tests/native/fake_kernels.cpp classeq2_b200/csrc/{index_build,host_api,host_pack,host_pool}.cpp oracle/classeq_oracle.cpp -o host_floor
 //   CLS_HOST_THREADS=4 ./host_floor 10000000
 #include <atomic>
